@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- sparse_mm forward+backward throughput on B200 (BASELINE.json's metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 2] [--impl reference] [--dump-outputs DIR]
 
 One step = one forward + backward of ``sparse_mm(A, B)`` (C = A B; grad_A by SDDMM; grad_B = A^T G)
 over one batch of synthetic input.  Default workload = BASELINE.json configs[1] ("config 2"): batched
@@ -19,6 +19,10 @@ Prints ONE JSON line (rank 0).  `value` = nnz/s with inputs resident in HBM; `e2
 through the public API from pinned HOST buffers (H2D of A, B, G and D2H of C, grad_A, grad_B inside
 the timed region); `roofline` = the dominant kernel against the measured HBM copy bandwidth;
 `cpu_baseline` = the reference's CPU data flow (oracle/reference_port.py) on this host's cores.
+
+`--dump-outputs DIR` writes what the timed region's last step computed (C, grad_A values, grad_B) as
+DIR/<name>.npy, so that two builds run with the same arguments (hence the same seeded inputs) can be compared
+output for output.
 """
 from __future__ import annotations
 
@@ -31,6 +35,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -112,6 +117,26 @@ def problem_stats(A, K):
     alg = W.algorithmic_bytes(batch, n, m, nnz_total // batch, K, s_v, s_i, coo=coo)
     return dict(batch=batch, n=n, m=m, nnz=nnz_total, K=K, s_v=s_v, s_i=s_i, alg=alg,
                 flops=6 * nnz_total * K, gather_bytes_per_pass=nnz_total * K * s_v)
+
+
+DUMP_BYTES_PER_OUTPUT = 16 << 20  # three outputs: at most 48 MiB per dump
+
+
+def dump_outputs(outputs: dict, out_dir: str, max_bytes: int = DUMP_BYTES_PER_OUTPUT) -> None:
+    """Write every tensor of `outputs` as out_dir/<name>.npy: float64 stays float64, other float types become float32.
+    A tensor larger than `max_bytes` is cut to a fixed sample of its rows (the last dimension kept whole; elements of
+    a 1-D tensor), drawn with numpy's default_rng(0) from its shape alone, so two runs with the same arguments write
+    the same positions."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        t = t.detach()
+        t = t.double() if t.dtype == torch.float64 else t.float()
+        if t.numel() * t.element_size() > max_bytes:
+            t = t.reshape(-1, t.shape[-1]) if t.dim() > 1 else t
+            keep = max(max_bytes // (t[0].numel() * t.element_size()), 1)
+            rows = np.sort(np.random.default_rng(0).choice(t.shape[0], keep, replace=False))
+            t = t[torch.from_numpy(rows).to(t.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
 
 
 # ----------------------------------------------------------------------------- clocks sampler
@@ -328,15 +353,26 @@ def reference_methodology_ms(A, B, op, repeats=10):
     return res
 
 
+def _positive_int(text: str) -> int:
+    value = int(text)
+    if value < 1:
+        raise argparse.ArgumentTypeError(f"must be at least 1, got {value}")
+    return value
+
+
 def main():
     _route_library_chatter_to_stderr()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=_positive_int, default=50, help="timed steps of every timed region (e2e included)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--config", default="2", choices=sorted(CONFIGS))
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
-    ap.add_argument("--e2e-steps", type=int, default=10)
+    ap.add_argument("--e2e-steps", type=_positive_int, default=None, help="timed steps of the e2e leg (default: --steps)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the timed region's last-step outputs (C, grad_A values, grad_B; rank 0's share at N > 1) "
+                         f"as DIR/<name>.npy; an output over {DUMP_BYTES_PER_OUTPUT >> 20} MiB is cut to a fixed seeded "
+                         "sample of its rows")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--sharding", default="k", choices=["rows", "k"],
@@ -436,12 +472,23 @@ def main():
     else:
         op = D.sparse_mm_k_sharded if k_sharded else sparse_mm
 
+    last_C = [None]
+
     def step():
         A.grad = None
         B.grad = None
         C = op(A, B)
         C.backward(G)
+        # detached: a reference to C itself would keep this step's autograd graph alive, and a CUDA graph capture on
+        # the side stream fails while it is.  Inside a capture this is the static output every replay rewrites.
+        last_C[0] = C.detach()
         return C
+
+    def step_outputs():
+        """What a caller of the step receives from its latest run (the captured one's tensors after graph replays);
+        grad_A values flattened in storage order, so that a sample of them is drawn per entry, not per batch item."""
+        gA = A.grad.values() if A.grad.layout == torch.sparse_csr else A.grad._values()
+        return {"C": last_C[0], "grad_A_values": gA.reshape(-1), "grad_B": B.grad}
 
     def barrier():
         torch.cuda.synchronize()
@@ -514,6 +561,7 @@ def main():
     # region A: eager steps through the public op, with per-kernel CUDA events (roofline) and the host enqueue time
     eager_total, host_ms, clocks, ksum, launches = timed_region(step, True)
     timed = {"region": "eager", "ms_total": eager_total}
+    timed_outputs = step_outputs() if args.dump_outputs else None
     # region B: the same step replayed from a CUDA graph (fixed pattern, fixed shapes): no host work between kernels
     graph_note = None
     if (row_sharded or k_sharded) and not args.no_graph:
@@ -539,6 +587,7 @@ def main():
             if g_total <= eager_total:
                 timed = {"region": "cuda_graph", "ms_total": g_total}
                 clocks, launches = g_clocks, graph_launches * args.steps
+                timed_outputs = step_outputs() if args.dump_outputs else None
         except Exception as exc:  # noqa: BLE001 -- capture not possible (e.g. a collective that refuses capture): eager stands
             graph_note = {"unavailable": f"{type(exc).__name__}: {exc}"[:200]}
             torch.cuda.synchronize()
@@ -547,6 +596,9 @@ def main():
         "CUDA-graph replay of the step (pattern and shapes fixed); per-kernel durations and host enqueue time from the "
         "eager region run beside it (same K steps, same work)" if timed["region"] == "cuda_graph" else
         "eager steps through the public op")
+    if timed_outputs is not None and rank == 0:
+        dump_outputs(timed_outputs, args.dump_outputs)
+    timed_outputs = None
     if dist is not None:
         t = torch.tensor([ms_total, eager_total, host_ms], device=dev, dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -602,7 +654,7 @@ def main():
     # ---- e2e: same step through the public API from pinned host buffers
     e2e = None
     if not args.no_e2e:
-        e2e = run_e2e(A.detach(), B.detach(), G, args.e2e_steps, dev, dist, op)
+        e2e = run_e2e(A.detach(), B.detach(), G, args.e2e_steps or args.steps, dev, dist, op)
         e2e["value"] = (nnz_all / (e2e.pop("ms_per_step_max") * 1e-3))
 
     cpu_base = None

@@ -235,6 +235,35 @@ def test_bench_stdout_carries_only_the_json_line(tmp_path):
     assert "NCCL version banner" in r.stderr and "python-level chatter" in r.stderr
 
 
+def test_bench_dump_outputs_is_bounded_and_repeatable(tmp_path):
+    """--dump-outputs: float32 / float64 files, whole when small, otherwise the same seeded sample of whole rows (or
+    elements of a 1-D output) on every run, within the per-output byte bound."""
+    import os
+    import sys
+
+    import numpy as np
+    import torch
+
+    sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+    import bench
+
+    g = torch.Generator().manual_seed(0)
+    outs = {"C": torch.rand(3, 50, 8, generator=g), "grad_A_values": torch.rand(1000, generator=g, dtype=torch.float64),
+            "grad_B": torch.rand(4, 6, generator=g).to(torch.bfloat16)}
+    for run in ("a", "b"):
+        bench.dump_outputs(outs, str(tmp_path / run), max_bytes=1024)
+    for name, t in outs.items():
+        a, b = np.load(tmp_path / "a" / f"{name}.npy"), np.load(tmp_path / "b" / f"{name}.npy")
+        assert np.array_equal(a, b) and a.nbytes <= 1024
+        assert a.dtype == (np.float64 if t.dtype == torch.float64 else np.float32)
+    assert np.array_equal(np.load(tmp_path / "a" / "grad_B.npy"), outs["grad_B"].float().numpy())  # small: whole
+    C = np.load(tmp_path / "a" / "C.npy")
+    rows = outs["C"].reshape(-1, 8).numpy()
+    assert C.shape == (1024 // 32, 8) and all((rows == r).all(axis=1).any() for r in C)
+    gA = np.load(tmp_path / "a" / "grad_A_values.npy")
+    assert gA.shape == (128,) and np.isin(gA, outs["grad_A_values"].numpy()).all()
+
+
 def test_sort_rows_by_length_is_a_row_permutation_with_snake_blocks():
     """Host-side layout optimisation of the cached transpose (pure index arithmetic, runs on any device): rows are
     permuted inside blocks of 64, alternately longest-first / shortest-first, entries of a row stay together and in
