@@ -38,7 +38,7 @@
 extern "C" {
 #endif
 
-#define TSGU_ABI_VERSION 1
+#define TSGU_ABI_VERSION 2
 
 #if defined(__GNUC__)
 #define TSGU_API __attribute__((visibility("default")))
@@ -133,28 +133,6 @@ TSGU_API int tsgu_sddmm_csr(const void* rowptr, const void* colind, const void* 
                    int val_dtype, int idx_dtype, int algo,
                    void* workspace, size_t workspace_bytes, void* stream);
 TSGU_API size_t tsgu_sddmm_workspace_bytes(int64_t batch, int64_t n, int64_t nnz_total, int algo);
-
-/* ------------------------------------------------------------------------------------
- * Split-row mode for badly skewed row lengths (one matrix, batch = 1): `vrowptr` (n_virtual + 1) cuts
- * every row longer than a bound into consecutive pieces ("virtual rows") over the SAME colind / vals
- * arrays, so the persistent row-tile kernels see rows of bounded length and stay balanced.
- *   SpMM : row_map[v] >= 0 -> virtual row v is row row_map[v] of C (it was not cut);
- *          row_map[v] <  0 -> it is piece ~row_map[v]: its partial sum is written to `partials`
- *          (accumulator precision: fp32, fp64 for fp64; K per piece) and tsgu_sum_row_pieces adds the
- *          pieces of each cut row up in order (rows[i] = the row, ptr[i]..ptr[i+1] = its pieces).
- *   SDDMM: row_map[v] = the row of G that virtual row v belongs to; out[] is indexed by entry as usual.
- * Requires 128-bit addressable dense operands (returns TSGU_ERR_SHAPE otherwise).
- * ---------------------------------------------------------------------------------- */
-TSGU_API int tsgu_spmm_csr_split(const void* vrowptr, const void* colind, const void* vals, const void* perm,
-                        const void* row_map, const void* B, void* C, void* partials,
-                        int64_t n_virtual, int64_t m, int64_t K, int64_t nnz_total, int64_t b_rs, int64_t ldc,
-                        int val_dtype, int idx_dtype, void* stream);
-TSGU_API int tsgu_sddmm_csr_split(const void* vrowptr, const void* colind, const void* out_index, const void* row_map,
-                         const void* G, const void* B, void* out,
-                         int64_t n_virtual, int64_t m, int64_t K, int64_t nnz_total, int64_t g_rs, int64_t b_rs,
-                         int val_dtype, int idx_dtype, void* stream);
-TSGU_API int tsgu_sum_row_pieces(const void* partials, const void* rows, const void* ptr, int64_t num_rows, int64_t K,
-                        void* C, int64_t ldc, int val_dtype, int idx_dtype, void* stream);
 
 /* Order-agnostic COO variant: row/col are int64 arrays of length nnz (torch COO indices,
  * sparse_matmul.py:184-185); out[e] = <G[row[e],:], B[col[e],:]>.  Also the kernel the
@@ -269,13 +247,14 @@ TSGU_API int tsgu_pack_dense_add(const void* src, const void* add, const void* r
  * for the compute entry points).  The compute kernels need K * sizeof(value) in {64, 128, 256}
  * bytes and 16-byte aligned dense rows; `out` of the SDDMM is written exactly like tsgu_sddmm_csr; the SpMM writes element
  * (r, k) of item t at C + t*c_bs + r*ldc + k*c_cs: c_cs == 1 is the row-major result of tsgu_spmm_csr, ldc == 1 a
- * column-major one (grad_B in the layout of a column-major B, without a separate layout pass). */
+ * column-major one (grad_B in the layout of a column-major B, without a separate layout pass).  The SpMM reads `vals` in
+ * pattern order (entry e has value vals[e]); callers whose values are permuted run tsgu_gather_values first. */
 TSGU_API int tsgu_window_limits(int* tile_rows_max, int* entries_max, int* window_rows, int* runs_max);
 TSGU_API int tsgu_window_plan(const void* rowptr, const void* colind, int64_t batch, int64_t n,
                      int64_t rowptr_bstride, int64_t nnz_bstride, int idx_dtype, int tile_rows,
                      void* lcol_out, void* desc_out, void* stats_out, void* stream);
 TSGU_API int tsgu_spmm_window(const void* rowptr, const void* lcol, const void* desc, const void* vals,
-                     const void* perm, const void* B, void* C, int64_t batch, int64_t n, int64_t K,
+                     const void* B, void* C, int64_t batch, int64_t n, int64_t K,
                      int64_t rowptr_bstride, int64_t nnz_bstride, int64_t nnz_len, int tile_rows,
                      int64_t b_bs, int64_t b_rs, int64_t c_bs, int64_t ldc, int64_t c_cs, int val_dtype,
                      int idx_dtype, void* stream);

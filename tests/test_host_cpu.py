@@ -120,7 +120,7 @@ def test_header_binding_and_library_agree():
     L = nat.lib()  # sets argtypes for every symbol; AttributeError if one is missing
     for name in declared:
         assert hasattr(L, name)
-    assert L.tsgu_version() == 1
+    assert L.tsgu_version() == 2
     assert L.tsgu_error_string(-3).decode().startswith("tsgu: workspace")
     assert nat.launch_count() >= 0
     out = subprocess.run(["nm", "-D", "--defined-only", nat.LIB_PATH], capture_output=True, text=True).stdout

@@ -181,13 +181,9 @@ def test_batched_csr_window():
     _check_against_oracle(A, 32, torch.float32)
 
 
-@pytest.mark.parametrize("perm_in_kernel", [False, True])
-def test_uncoalesced_coo_stencil_window(perm_in_kernel, monkeypatch):
-    """COO in shuffled storage order: the flat CSR carries a value permutation (pre-gathered, or read inside the
-    kernel with TSGU_B200_WINDOW_PERM=1)."""
-    from torchsparsegradutils_b200 import _ops
-
-    monkeypatch.setattr(_ops, "_WINDOW_PERM_IN_KERNEL", perm_in_kernel)
+def test_uncoalesced_coo_stencil_window():
+    """COO in shuffled storage order: the flat CSR carries a value permutation (values pre-gathered into pattern
+    order before the window SpMM)."""
     Ac = W.stencil27_csr(12, torch.float32, torch.int32, DEV, seed=3).to_sparse_coo()
     idx, v = Ac._indices(), Ac._values()
     sh = torch.randperm(v.numel(), generator=torch.Generator().manual_seed(1)).to(DEV)

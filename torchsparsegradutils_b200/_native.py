@@ -21,7 +21,6 @@ F32, F64, BF16 = 0, 1, 2
 I32, I64 = 0, 1
 ALGO_AUTO, ALGO_ROWSPLIT, ALGO_MERGE = 0, 1, 2
 ALGO_FLAG_KSLICE = 0x100  # OR-ed into algo for tsgu_spmm_csr: uniform rows, K may be cut into L2-resident slices
-ALGO_SPLIT = 3  # host-side choice only: split long rows into virtual rows (tsgu_*_csr_split entry points)
 
 VAL_DTYPES = {torch.float32: F32, torch.float64: F64, torch.bfloat16: BF16}
 IDX_DTYPES = {torch.int32: I32, torch.int64: I64}
@@ -42,9 +41,6 @@ _SIGNATURES = {
     "tsgu_spmm_workspace_bytes": (_Z, [_L, _L, _L, _L, _I, _I]),
     "tsgu_sddmm_csr": (_I, [_P, _P, _P, _P, _P, _P, _L, _L, _L, _L, _L, _L, _L, _L, _L, _L, _L, _L, _L, _I, _I, _I, _P, _Z, _P]),
     "tsgu_sddmm_workspace_bytes": (_Z, [_L, _L, _L, _I]),
-    "tsgu_spmm_csr_split": (_I, [_P, _P, _P, _P, _P, _P, _P, _P, _L, _L, _L, _L, _L, _L, _I, _I, _P]),
-    "tsgu_sddmm_csr_split": (_I, [_P, _P, _P, _P, _P, _P, _P, _L, _L, _L, _L, _L, _L, _I, _I, _P]),
-    "tsgu_sum_row_pieces": (_I, [_P, _P, _P, _L, _L, _P, _L, _I, _I, _P]),
     "tsgu_sddmm_coo": (_I, [_P, _P, _P, _P, _P, _L, _L, _L, _L, _L, _L, _I, _P]),
     "tsgu_coo_sort": (_I, [_P, _I, _L, _L, _P, _I, _P, _P, _I, _P, _Z, _P]),
     "tsgu_coo_sort_workspace_bytes": (_Z, [_I, _L, _I]),
@@ -62,7 +58,7 @@ _SIGNATURES = {
     "tsgu_pack_dense_add": (_I, [_P, _P, _P, _P, _L, _L, _L, _L, _L, _L, _L, _L, _L, _L, _L, _I, _P]),
     "tsgu_window_limits": (_I, [_P, _P, _P, _P]),
     "tsgu_window_plan": (_I, [_P, _P, _L, _L, _L, _L, _I, _I, _P, _P, _P, _P]),
-    "tsgu_spmm_window": (_I, [_P, _P, _P, _P, _P, _P, _P, _L, _L, _L, _L, _L, _L, _I, _L, _L, _L, _L, _L, _I, _I, _P]),
+    "tsgu_spmm_window": (_I, [_P, _P, _P, _P, _P, _P, _L, _L, _L, _L, _L, _L, _I, _L, _L, _L, _L, _L, _I, _I, _P]),
     "tsgu_sddmm_window": (_I, [_P, _P, _P, _P, _P, _P, _P, _L, _L, _L, _L, _L, _L, _I, _L, _L, _L, _L, _I, _I, _P]),
 }
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)

@@ -174,16 +174,6 @@ def _strides(x: torch.Tensor):
     return (bs if x.shape[0] > 1 else 0, rs if x.shape[1] > 1 else 0, cs if x.shape[2] > 1 else 1)
 
 
-def _split_ready(pat: CsrPattern, *dense: torch.Tensor) -> bool:
-    """Split-row mode needs the persistent-tile kernels: 128-bit addressable operands, K <= 128 vectors."""
-    if pat.split is None or pat.batch != 1:
-        return False
-    for x in dense:
-        if not _vector_ready(x) or x.shape[-1] // _VEC_ELEMS[x.dtype] > 128:
-            return False
-    return True
-
-
 _L2_BYTES = {}
 
 
@@ -194,14 +184,7 @@ def _l2_bytes(dev: torch.device) -> int:
     return _L2_BYTES[key]
 
 
-def wants_pregather(pat: CsrPattern) -> bool:
-    """True when spmm() would first put the values into the pattern's own order (one streaming pass)."""
-    return pat.perm is not None and pat.nnz_total >= _PREGATHER_MIN_NNZ and pat.algo != nat.ALGO_SPLIT
-
-
-_KSLICE_SORTED = os.environ.get("TSGU_B200_KSLICE_SORTED", "0") == "1"
 _WINDOW_ROW_BYTES = (64, 128, 256)  # dense row widths the column-window kernels are built for (csrc/window.cu)
-_WINDOW_PERM_IN_KERNEL = os.environ.get("TSGU_B200_WINDOW_PERM", "0") == "1"
 
 
 def _window_for(pat: CsrPattern, algo: int, *dense: torch.Tensor) -> Optional[WindowPlan]:
@@ -217,7 +200,7 @@ def _window_for(pat: CsrPattern, algo: int, *dense: torch.Tensor) -> Optional[Wi
 
 
 def _spmm_window(pat: CsrPattern, wp: WindowPlan, vals: torch.Tensor, dense: torch.Tensor, tag: str,
-                 vals_in_pattern_order: bool, out_strides=None) -> torch.Tensor:
+                 out_strides=None) -> torch.Tensor:
     dev = dense.device
     K = dense.shape[-1]
     colmajor = out_strides is not None and tuple(out_strides) == (pat.n * K, 1, pat.n) and K > 1 and pat.n > 1
@@ -225,15 +208,13 @@ def _spmm_window(pat: CsrPattern, wp: WindowPlan, vals: torch.Tensor, dense: tor
         out = torch.empty_strided((pat.batch, pat.n, K), (pat.n * K, 1, pat.n), dtype=dense.dtype, device=dev)
     else:
         out = torch.empty((pat.batch, pat.n, K), dtype=dense.dtype, device=dev)
-    perm = None if vals_in_pattern_order else pat.perm
-    if perm is not None and not _WINDOW_PERM_IN_KERNEL:
+    if pat.perm is not None:
         with _timer(tag + "_gather", dev):
-            vals = gather_values(vals.reshape(-1), perm)
-        perm = None
+            vals = gather_values(vals.reshape(-1), pat.perm)
     bs, rs, _ = _strides(dense)
     with _on(dev), _timer(tag, dev):
         nat.check(nat.lib().tsgu_spmm_window(nat.ptr(pat.rowptr), nat.ptr(wp.lcol), nat.ptr(wp.desc), nat.ptr(vals),
-                                             nat.ptr(perm), dense.data_ptr(), out.data_ptr(), pat.batch, pat.n, K,
+                                             dense.data_ptr(), out.data_ptr(), pat.batch, pat.n, K,
                                              pat.rowptr_bstride, pat.nnz_bstride, pat.colind.numel(), wp.tile_rows,
                                              bs, rs if pat.m > 1 else K, pat.n * K, 1 if colmajor else K,
                                              pat.n if colmajor else 1, nat.val_enum(dense.dtype), pat.idx,
@@ -242,31 +223,25 @@ def _spmm_window(pat: CsrPattern, wp: WindowPlan, vals: torch.Tensor, dense: tor
 
 
 def spmm(pat: CsrPattern, vals: torch.Tensor, dense: torch.Tensor, algo: Optional[int] = None,
-         tag: str = "spmm", vals_in_pattern_order: bool = False, out_strides=None) -> torch.Tensor:
+         tag: str = "spmm", out_strides=None) -> torch.Tensor:
     """out[t] = A[t] @ dense[t]; dense is (batch, m, K) (any strides); returns contiguous (batch, n, K).
-    `vals_in_pattern_order`: `vals` were already gathered through `pat.perm` by the caller (gather_values).
     `out_strides`: a layout the caller would like the (batch, n, K) result in; honoured where a kernel can write it
     directly (column-major items from the column-window kernels), otherwise the result is contiguous and the caller
     re-strides it."""
     algo = pat.algo if algo is None else algo
-    if algo == nat.ALGO_SPLIT:
-        d3 = prepare_dense(_as3d(dense))
-        if _split_ready(pat, d3):
-            return _spmm_split(pat, vals, d3, tag)
-        algo = nat.ALGO_MERGE  # scalar / oversized K: the merge-path (or row-split) kernels take it
     dense = prepare_dense(_as3d(dense))
     K = dense.shape[-1]
     if pat.batch * pat.n * K and pat.nnz_total:
         wp = _window_for(pat, algo, dense)
         if wp is not None:
-            return _spmm_window(pat, wp, vals, dense, tag, vals_in_pattern_order, out_strides)
+            return _spmm_window(pat, wp, vals, dense, tag, out_strides)
     out = torch.empty((pat.batch, pat.n, K), dtype=dense.dtype, device=dense.device)
     if out.numel() == 0:
         return out
     dev = dense.device
     L = nat.lib()
     vdt = nat.val_enum(dense.dtype)
-    perm = None if vals_in_pattern_order else pat.perm
+    perm = pat.perm
     if perm is not None and (pat.nnz_total >= _PREGATHER_MIN_NNZ or pat.padded):
         # one streaming pass that puts the values in the structure's own order is cheaper than a
         # divergent 4-byte gather per entry inside the bandwidth-critical SpMM (0.37 -> 0.25+0.03 ms on config 2)
@@ -274,7 +249,7 @@ def spmm(pat: CsrPattern, vals: torch.Tensor, dense: torch.Tensor, algo: Optiona
             vals = gather_values(vals.reshape(-1), perm)
         perm = None
     if (algo == nat.ALGO_AUTO and pat.m * K * dense.element_size() > (_l2_bytes(dev) * 3) // 5
-            and (pat.uniform_rows or (_KSLICE_SORTED and pat.row_map is not None))):
+            and pat.uniform_rows):
         algo |= nat.ALGO_FLAG_KSLICE  # dense operand exceeds L2 and the rows are uniform: L2-resident K slices
     if pat.row_map is not None:  # a transpose with length-sorted rows
         with _on(dev), _timer(tag, dev):
@@ -295,51 +270,10 @@ def spmm(pat: CsrPattern, vals: torch.Tensor, dense: torch.Tensor, algo: Optiona
     return out
 
 
-def _spmm_split(pat: CsrPattern, vals: torch.Tensor, dense: torch.Tensor, tag: str) -> torch.Tensor:
-    """SpMM over the virtual rows of a skewed pattern + ordered sum of the pieces of cut rows."""
-    sp = pat.split
-    dev = dense.device
-    K = dense.shape[-1]
-    out = torch.empty((1, pat.n, K), dtype=dense.dtype, device=dev)
-    acc_dtype = torch.float64 if dense.dtype == torch.float64 else torch.float32
-    partials = torch.empty((max(sp.num_pieces, 1), K), dtype=acc_dtype, device=dev)
-    L = nat.lib()
-    vdt = nat.val_enum(dense.dtype)
-    perm = pat.perm
-    if perm is not None and pat.nnz_total >= _PREGATHER_MIN_NNZ:
-        with _timer(tag + "_gather", dev):
-            vals = gather_values(vals.reshape(-1), perm)
-        perm = None
-    with _on(dev), _timer(tag, dev):
-        nat.check(L.tsgu_spmm_csr_split(nat.ptr(sp.vrowptr), nat.ptr(pat.colind), nat.ptr(vals), nat.ptr(perm),
-                                        nat.ptr(sp.row_map), dense.data_ptr(), out.data_ptr(), partials.data_ptr(),
-                                        sp.n_virtual, pat.m, K, pat.nnz_total, dense.stride(1) if dense.shape[1] > 1 else K, K,
-                                        vdt, pat.idx, nat.stream_ptr(dev)), "tsgu_spmm_csr_split")
-        if sp.num_pieces:
-            nat.check(L.tsgu_sum_row_pieces(partials.data_ptr(), nat.ptr(sp.cut_rows), nat.ptr(sp.cut_ptr),
-                                            sp.cut_rows.numel(), K, out.data_ptr(), K, vdt, pat.idx,
-                                            nat.stream_ptr(dev)), "tsgu_sum_row_pieces")
-    return out
-
-
 def sddmm(pat: CsrPattern, G: torch.Tensor, B: torch.Tensor, out_index: Optional[torch.Tensor], nnz_out: int,
           algo: Optional[int] = None) -> torch.Tensor:
     """values[dst(e)] = <G[t, r_e], B[t, c_e]> for every stored entry of the pattern."""
     algo = pat.algo if algo is None else algo
-    if algo == nat.ALGO_SPLIT:
-        G3, B3 = prepare_dense(_as3d(G)), prepare_dense(_as3d(B))
-        if nnz_out and _split_ready(pat, G3, B3):
-            sp = pat.split
-            out = torch.empty(nnz_out, dtype=B3.dtype, device=B3.device)
-            dev = B3.device
-            with _on(dev), _timer("sddmm", dev):
-                nat.check(nat.lib().tsgu_sddmm_csr_split(
-                    nat.ptr(sp.vrowptr), nat.ptr(pat.colind), nat.ptr(out_index), nat.ptr(sp.g_map), G3.data_ptr(),
-                    B3.data_ptr(), out.data_ptr(), sp.n_virtual, pat.m, B3.shape[-1], pat.nnz_total,
-                    G3.stride(1) if G3.shape[1] > 1 else G3.shape[-1], B3.stride(1) if B3.shape[1] > 1 else B3.shape[-1],
-                    nat.val_enum(B3.dtype), pat.idx, nat.stream_ptr(dev)), "tsgu_sddmm_csr_split")
-            return out
-        algo = nat.ALGO_MERGE
     G = prepare_dense(_as3d(G))
     B = prepare_dense(_as3d(B))
     out = torch.empty(nnz_out, dtype=B.dtype, device=B.device)

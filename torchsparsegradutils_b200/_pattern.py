@@ -84,8 +84,6 @@ def pattern_nbytes(p) -> int:
                 + (_tensor_bytes(p.out_index) if p.out_index is not p.csr.perm else 0))
     total = sum(_tensor_bytes(t) for t in (p.rowptr, p.colind, p.perm))
     total += sum(_tensor_bytes(t) for t in p.keep if isinstance(t, torch.Tensor) and t is not p.rowptr and t is not p.colind)
-    if p.split is not None:
-        total += sum(_tensor_bytes(t) for t in (p.split.vrowptr, p.split.row_map, p.split.g_map, p.split.cut_rows, p.split.cut_ptr))
     for extra in p.extras.values():
         if isinstance(extra, WindowPlan):
             extra = (extra.lcol, extra.desc)
@@ -152,7 +150,6 @@ class CsrPattern:
     nnz_total: int
     idx: int  # nat.I32 / nat.I64
     algo: int = nat.ALGO_AUTO  # kernel family chosen once per pattern from its row-length skew
-    split: Optional["SplitRows"] = None  # virtual-row view of a skewed pattern (algo == ALGO_SPLIT)
     keep: tuple = ()  # tensors whose storage must outlive this pattern (cache-key owners)
     row_map: Optional[torch.Tensor] = None  # rows were permuted: CSR row s of item t is output row row_map[t*n + s]
     padded: bool = False  # perm holds -1 entries (explicit zeros): the values MUST go through gather_values, never the in-kernel perm path
@@ -207,45 +204,7 @@ class CsrPattern:
         return t
 
 
-@dataclass
-class SplitRows:
-    """Long rows cut into consecutive pieces of at most `bound` entries over the same colind / vals arrays."""
-
-    vrowptr: torch.Tensor   # (n_virtual + 1,)
-    row_map: torch.Tensor   # SpMM: >= 0 the row of C, < 0 piece ~x of a cut row
-    g_map: torch.Tensor     # SDDMM: row of G each virtual row belongs to
-    cut_rows: torch.Tensor  # rows that were cut
-    cut_ptr: torch.Tensor   # (len(cut_rows) + 1,) piece ranges
-    n_virtual: int
-    num_pieces: int
-
-
-def build_split_rows(rowptr: torch.Tensor, n: int, nnz: int, bound: int) -> SplitRows:
-    """One-off per pattern (a handful of torch ops, two host syncs for the sizes)."""
-    dev, idt = rowptr.device, rowptr.dtype
-    rp = rowptr.reshape(-1).long()
-    lens = rp[1:] - rp[:-1]
-    nv = ((lens + (bound - 1)) // bound).clamp_(min=1)
-    first_v = torch.cumsum(nv, 0) - nv
-    n_virtual = int(nv.sum())
-    row_of_v = torch.repeat_interleave(torch.arange(n, device=dev), nv)
-    j = torch.arange(n_virtual, device=dev) - first_v[row_of_v]
-    vrowptr = torch.empty(n_virtual + 1, dtype=torch.int64, device=dev)
-    vrowptr[:-1] = rp[:-1][row_of_v] + j * bound
-    vrowptr[-1] = nnz
-    cut = nv > 1
-    is_piece = cut[row_of_v]
-    pidx = torch.cumsum(is_piece.long(), 0) - 1
-    row_map = torch.where(is_piece, -1 - pidx, row_of_v)
-    cut_rows = torch.nonzero(cut).flatten()
-    cut_ptr = torch.zeros(cut_rows.numel() + 1, dtype=torch.int64, device=dev)
-    cut_ptr[1:] = torch.cumsum(nv[cut], 0)
-    return SplitRows(vrowptr.to(idt), row_map.to(idt), row_of_v.to(idt), cut_rows.to(idt), cut_ptr.to(idt), n_virtual,
-                     int(is_piece.sum()))
-
-
-_ALGO_ENV = {"auto": None, "rowsplit": nat.ALGO_ROWSPLIT, "merge": nat.ALGO_MERGE, "split": nat.ALGO_SPLIT}
-_SKEWED_ALGO = nat.ALGO_MERGE  # what the skew heuristic picks (ALGO_MERGE or ALGO_SPLIT)
+_ALGO_ENV = {"auto": None, "rowsplit": nat.ALGO_ROWSPLIT, "merge": nat.ALGO_MERGE}
 
 
 def choose_algo(rowptr: torch.Tensor, batch: int, n: int, nnz_total: int) -> int:
@@ -259,18 +218,16 @@ def choose_algo(rowptr: torch.Tensor, batch: int, n: int, nnz_total: int) -> int
     kernels and its rank took 25 ms per step).  One host sync per new pattern.  ``TSGU_B200_ALGO=auto|rowsplit|merge`` overrides the heuristic (benchmarking only).
     """
     forced = _ALGO_ENV.get(os.environ.get("TSGU_B200_ALGO", "auto").lower())
-    if forced is not None and forced != nat.ALGO_SPLIT:
+    if forced is not None:
         return forced
     if batch != 1 or nnz_total == 0 or n == 0:
         return nat.ALGO_AUTO
-    if forced is not None:
-        return forced
     flat = rowptr.reshape(-1)  # batch == 1: torch batched CSR keeps a leading dim of 1
     return _algo_from_max_row(nat.host_read((flat[1:] - flat[:-1]).max())[0], n, nnz_total)
 
 
 def _algo_from_max_row(max_row: int, n: int, nnz_total: int) -> int:
-    return _SKEWED_ALGO if (max_row > 256 and max_row > 16 * (nnz_total / n)) else nat.ALGO_AUTO
+    return nat.ALGO_MERGE if (max_row > 256 and max_row > 16 * (nnz_total / n)) else nat.ALGO_AUTO
 
 
 def _needs_row_stats(batch: int, n: int, nnz_total: int) -> bool:
@@ -429,7 +386,7 @@ def _build_transpose(p: CsrPattern) -> CsrPattern:
         # apply -- later, if the pattern turns out to be reused (CsrPattern.transpose).  No further host sync then: the
         # padded size came with the verdicts above.
         patT.extras["layout_pending"] = padded_total
-    return _with_split(patT)
+    return patT
 
 
 _LAYOUT_AFTER_USES = int(os.environ.get("TSGU_B200_LAYOUT_AFTER_USES", "2"))
@@ -441,12 +398,11 @@ def _optimise_layout(patT: CsrPattern) -> CsrPattern:
     (skipped if the padding would overflow a 32-bit rowptr).  Returns a new pattern; `patT` is left untouched for
     whoever still holds it."""
     padded_total = patT.extras["layout_pending"]
-    rowptrT, colindT, permT, row_map = patT.rowptr, patT.colind, patT.perm, None
+    rowptrT, colindT, permT = patT.rowptr, patT.colind, patT.perm
     cur = torch.cuda.current_stream(patT.device)
     for t in (rowptrT, colindT, permT):
         t.record_stream(cur)  # the caller drops patT right after; it may have been built under another stream
-    if _SORT_ROWS:
-        rowptrT, colindT, permT, row_map = _sort_rows_by_length(rowptrT, colindT, permT, patT.batch, patT.n)
+    rowptrT, colindT, permT, row_map = _sort_rows_by_length(rowptrT, colindT, permT, patT.batch, patT.n)
     if (patT.idx == nat.I64 or padded_total < _I32_MAX) and padded_total > patT.nnz_total:
         rowptrT, colindT, permT = _pad_rows(rowptrT, colindT, permT, _ROW_PAD, padded_total)
     new = CsrPattern(rowptrT, colindT, permT, patT.batch, patT.n, patT.m, patT.n, 0, permT.numel(), patT.idx,
@@ -454,19 +410,6 @@ def _optimise_layout(patT: CsrPattern) -> CsrPattern:
     new.extras["window"] = None
     new._uniform = patT._uniform
     return new
-
-
-def _split_bound() -> int:
-    return int(os.environ.get("TSGU_B200_SPLIT_BOUND", "128"))
-
-
-def _with_split(pat: CsrPattern) -> CsrPattern:
-    if pat.algo == nat.ALGO_SPLIT and pat.batch == 1:
-        pat.split = build_split_rows(pat.rowptr, pat.n, pat.nnz_total, _split_bound())
-    return pat
-
-
-_SORT_ROWS = os.environ.get("TSGU_B200_SORT_ROWS", "1") != "0"
 
 
 _SORT_BLOCK = 64  # rows per sorting block: a multiple of the rows one pass of a CTA's lane groups covers (32 or 64)
@@ -606,8 +549,8 @@ def csr_pattern(A: torch.Tensor) -> CsrPattern:
     nnz_item = col_c.shape[-1]
     idx = nat.idx_enum(crow.dtype)
     algo, plan, _, max_row = _analyse(crow_c, col_c, batch, n, m, n + 1, nnz_item, batch * nnz_item, idx)
-    pat = _with_split(CsrPattern(crow_c, col_c, None, batch, n, m, n + 1, nnz_item, batch * nnz_item, idx, algo=algo,
-                                 keep=(crow, col)))
+    pat = CsrPattern(crow_c, col_c, None, batch, n, m, n + 1, nnz_item, batch * nnz_item, idx, algo=algo,
+                     keep=(crow, col))
     pat._uniform = _uniform_from(max_row, batch * n, batch * nnz_item)
     pat.extras["window"] = plan
     pat.cache_key = key
@@ -662,7 +605,7 @@ def _coo_to_flat_csr(indices: torch.Tensor, batch: int, n: int, m: int, perm: Op
                                             nat.ptr(rowptr), nat.ptr(colind), idx, nat.stream_ptr(dev)),
                   "tsgu_coo_to_csr")
     algo, plan, _, max_row = _analyse(rowptr, colind, batch, n, m, n, 0, nnz, idx)
-    pat = _with_split(CsrPattern(rowptr, colind, perm, batch, n, m, n, 0, nnz, idx, algo=algo, keep=keep))
+    pat = CsrPattern(rowptr, colind, perm, batch, n, m, n, 0, nnz, idx, algo=algo, keep=keep)
     pat._uniform = _uniform_from(max_row, batch * n, nnz)
     pat.extras["window"] = plan
     return pat

@@ -123,21 +123,6 @@ __device__ __forceinline__ void store_vec(V* p, const typename VT<V>::Acc (&a)[E
   }
 }
 
-// 128-bit dense-row gather.  TSGU_GATHER_NO_L1=1 (build-time experiment) asks the load not to allocate in L1:
-// with uniformly random columns a B row is practically never re-used out of L1.
-#ifndef TSGU_GATHER_NO_L1
-#define TSGU_GATHER_NO_L1 0
-#endif
-__device__ __forceinline__ uint4 ldg_gather(const uint4* p) {
-#if TSGU_GATHER_NO_L1
-  uint4 v;
-  asm("ld.global.nc.L1::no_allocate.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));
-  return v;
-#else
-  return __ldg(p);
-#endif
-}
-
 // scalar value load as accumulator type
 template <typename V>
 __device__ __forceinline__ typename VT<V>::Acc load_scalar(const V* p) {

@@ -412,39 +412,9 @@ __global__ void __launch_bounds__(256) pack_dense_kernel(const V* __restrict__ s
   }
 }
 
-// C[rows[i], :] = sum of partials[k, :] for k in [ptr[i], ptr[i+1]), in order (deterministic).  One thread per
-// (cut row, column): coalesced along K, a short sequential loop over the pieces.
-template <typename V, typename I>
-__global__ void sum_row_pieces_kernel(const typename VT<V>::Acc* __restrict__ partials, const I* __restrict__ rows,
-                                      const I* __restrict__ ptr, int64_t num_rows, int64_t K, V* __restrict__ C,
-                                      int64_t ldc) {
-  using Acc = typename VT<V>::Acc;
-  const int64_t total = num_rows * K;
-  for (int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (int64_t)gridDim.x * blockDim.x) {
-    const int64_t i = t / K, k = t - i * K;
-    Acc a = Acc(0);
-    for (int64_t q = (int64_t)ptr[i]; q < (int64_t)ptr[i + 1]; ++q) a += partials[q * K + k];
-    C[(int64_t)rows[i] * ldc + k] = VT<V>::from_acc(a);
-  }
-}
-
 }  // namespace tsgu
 
 using namespace tsgu;
-
-extern "C" int tsgu_sum_row_pieces(const void* partials, const void* rows, const void* ptr, int64_t num_rows, int64_t K,
-                                   void* C, int64_t ldc, int val_dtype, int idx_dtype, void* stream) {
-  if (num_rows < 0 || K < 0) return TSGU_ERR_SHAPE;
-  if (num_rows == 0 || K == 0) return 0;
-  cudaStream_t s = as_stream(stream);
-  TSGU_DISPATCH_VAL(val_dtype, TSGU_DISPATCH_IDX(idx_dtype, {
-    sum_row_pieces_kernel<V, I><<<blocks_for(num_rows * K, 256), 256, 0, s>>>(
-        (const typename VT<V>::Acc*)partials, (const I*)rows, (const I*)ptr, num_rows, K, (V*)C, ldc);
-    count_launch();
-  }));
-  return launch_status();
-}
-
 
 extern "C" size_t tsgu_coo_sort_workspace_bytes(int ndim, int64_t nnz, int perm_dtype) {
   (void)ndim;

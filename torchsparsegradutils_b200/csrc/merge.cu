@@ -23,9 +23,6 @@
 #ifndef TSGU_MERGE_SDDMM_MINB
 #define TSGU_MERGE_SDDMM_MINB 3
 #endif
-#ifndef TSGU_MERGE_NARROW
-#define TSGU_MERGE_NARROW 1  // 8-lane groups with 2-4 vectors per lane, as the tile kernels (config 4: 9.7 -> 9.2 ms)
-#endif
 #ifndef TSGU_MERGE_LOADS
 #define TSGU_MERGE_LOADS 16  // 128-bit dense-row loads in flight per lane (SpMM)
 #endif
@@ -482,15 +479,10 @@ int spmm_merge_dispatch(const I* rowptr, const I* colind, const V* vals, const I
               : launch_spmm_merge<V, I, LPR_, VPL_, false>(rowptr, colind, vals, perm, B, C, rows, K, nnz, b_rs, ldc, ws, ws_bytes, s)
   if (kv <= 4) TSGU_MERGE(4, 1);
   if (kv <= 8) TSGU_MERGE(8, 1);
-#if TSGU_MERGE_NARROW
+  // 8-lane groups with 2-4 vectors per lane, as the tile kernels (config 4: 9.7 ms with 16/32-lane groups, 9.2 ms)
   if (kv <= 16) TSGU_MERGE(8, 2);
   if (kv <= 32) TSGU_MERGE(8, 4);
   if (kv <= 64) TSGU_MERGE(16, 4);
-#else
-  if (kv <= 16) TSGU_MERGE(16, 1);
-  if (kv <= 32) TSGU_MERGE(32, 1);
-  if (kv <= 64) TSGU_MERGE(32, 2);
-#endif
   TSGU_MERGE(32, 4);
 #undef TSGU_MERGE
 }
@@ -768,15 +760,9 @@ int sddmm_merge_dispatch(const I* rowptr, const I* colind, const I* out_index, c
   const int64_t kv = K / EPVF;
   if (kv <= 4) return launch_sddmm_merge<V, I, 4, 1>(p, ws, ws_bytes, s);
   if (kv <= 8) return launch_sddmm_merge<V, I, 8, 1>(p, ws, ws_bytes, s);
-#if TSGU_MERGE_NARROW
   if (kv <= 16) return launch_sddmm_merge<V, I, 8, 2>(p, ws, ws_bytes, s);
   if (kv <= 32) return launch_sddmm_merge<V, I, 8, 4>(p, ws, ws_bytes, s);
   if (kv <= 64) return launch_sddmm_merge<V, I, 16, 4>(p, ws, ws_bytes, s);
-#else
-  if (kv <= 16) return launch_sddmm_merge<V, I, 16, 1>(p, ws, ws_bytes, s);
-  if (kv <= 32) return launch_sddmm_merge<V, I, 32, 1>(p, ws, ws_bytes, s);
-  if (kv <= 64) return launch_sddmm_merge<V, I, 32, 2>(p, ws, ws_bytes, s);
-#endif
   return launch_sddmm_merge<V, I, 32, 4>(p, ws, ws_bytes, s);
 }
 

@@ -24,7 +24,6 @@ struct SddmmParams {
   int64_t rowptr_bstride, nnz_bstride;
   int64_t g_bs, g_rs, g_cs, b_bs, b_rs, b_cs;
   int accumulate;  // tile kernel: out[dst] += dot (K processed in L2-sized slices)
-  const I* row_map;  // split-row mode (tile kernel, batch == 1): G row of virtual row v is row_map[v]
 };
 
 // Reduce NB per-lane partials across the LPR lanes of a group with a halving butterfly.
@@ -220,8 +219,7 @@ __global__ void __launch_bounds__(256, TSGU_TILE_MINB(VPL)) sddmm_tile_kernel(co
       if (e0 >= e1) continue;
       // the row of the upstream gradient stays in registers for the whole row of A
       Acc g[VPL][EPV];
-      const int64_t grow = p.row_map ? (int64_t)p.row_map[c.r0 + lr] : (int64_t)(c.r0 + lr);
-      const V* Grow = p.G + c.item * p.g_bs + grow * p.g_rs;
+      const V* Grow = p.G + c.item * p.g_bs + (int64_t)(c.r0 + lr) * p.g_rs;
 #pragma unroll
       for (int w = 0; w < VPL; ++w) {
         Raw<V, EPV> raw = (EXACT || on[w]) ? raw_ldg<V, EPV>(Grow + (int64_t)(w * LPR + gl) * EPV) : raw_zero<V, EPV>();
@@ -251,7 +249,7 @@ __global__ void __launch_bounds__(256, TSGU_TILE_MINB(VPL)) sddmm_tile_kernel(co
               const char* brow = Bb + (uint64_t)cj * row_bytes;
 #pragma unroll
               for (int w = 0; w < VPL; ++w) {
-                if (EXACT || on[w]) b[u][w] = ldg_gather(reinterpret_cast<const uint4*>(brow + w * (LPR * 16)));
+                if (EXACT || on[w]) b[u][w] = __ldg(reinterpret_cast<const uint4*>(brow + w * (LPR * 16)));
                 else b[u][w] = make_uint4(0, 0, 0, 0);
               }
             }
@@ -275,7 +273,7 @@ __global__ void __launch_bounds__(256, TSGU_TILE_MINB(VPL)) sddmm_tile_kernel(co
               const char* brow = Bb + (uint64_t)cj * row_bytes;
 #pragma unroll
               for (int w = 0; w < VPL; ++w) {
-                if (j0 + u < cnt && (EXACT || on[w])) b[u][w] = ldg_gather(reinterpret_cast<const uint4*>(brow + w * (LPR * 16)));
+                if (j0 + u < cnt && (EXACT || on[w])) b[u][w] = __ldg(reinterpret_cast<const uint4*>(brow + w * (LPR * 16)));
                 else b[u][w] = make_uint4(0, 0, 0, 0);
               }
             }
@@ -355,19 +353,9 @@ static int sddmm_tile_dispatch(const SddmmParams<V, I>& p, int64_t nnz_total, cu
   const int64_t kv = p.K / EPVF;
   if (kv <= 4) return launch_sddmm_tile<V, I, 4, 1>(p, nnz_total, s);
   if (kv <= 8) return launch_sddmm_tile<V, I, 8, 1>(p, nnz_total, s);
-#if TSGU_LPR_CAP == 8
   if (kv <= 16) return launch_sddmm_tile<V, I, 8, 2>(p, nnz_total, s);
   if (kv <= 32) return launch_sddmm_tile<V, I, 8, 4>(p, nnz_total, s);
   if (kv <= 64) return launch_sddmm_tile<V, I, 16, 4>(p, nnz_total, s);
-#elif TSGU_LPR_CAP == 16
-  if (kv <= 16) return launch_sddmm_tile<V, I, 16, 1>(p, nnz_total, s);
-  if (kv <= 32) return launch_sddmm_tile<V, I, 16, 2>(p, nnz_total, s);
-  if (kv <= 64) return launch_sddmm_tile<V, I, 16, 4>(p, nnz_total, s);
-#else
-  if (kv <= 16) return launch_sddmm_tile<V, I, 16, 1>(p, nnz_total, s);
-  if (kv <= 32) return launch_sddmm_tile<V, I, 32, 1>(p, nnz_total, s);
-  if (kv <= 64) return launch_sddmm_tile<V, I, 32, 2>(p, nnz_total, s);
-#endif
   return launch_sddmm_tile<V, I, 32, 4>(p, nnz_total, s);
 }
 
@@ -501,32 +489,8 @@ extern "C" int tsgu_sddmm_csr(const void* rowptr, const void* colind, const void
     p.batch = batch; p.n = n; p.K = K;
     p.rowptr_bstride = rowptr_bstride; p.nnz_bstride = nnz_bstride;
     p.g_bs = g_bs; p.g_rs = g_rs; p.g_cs = g_cs; p.b_bs = b_bs; p.b_rs = b_rs; p.b_cs = b_cs;
-    p.accumulate = 0; p.row_map = nullptr;
+    p.accumulate = 0;
     return tsgu::sddmm_dispatch<V, I>(p, m, nnz_total, algo, workspace, workspace_bytes, tsgu::as_stream(stream));
-  }));
-  return 0;
-}
-
-extern "C" int tsgu_sddmm_csr_split(const void* vrowptr, const void* colind, const void* out_index, const void* row_map,
-                                    const void* G, const void* B, void* out, int64_t n_virtual, int64_t m, int64_t K,
-                                    int64_t nnz_total, int64_t g_rs, int64_t b_rs, int val_dtype, int idx_dtype,
-                                    void* stream) {
-  if (n_virtual < 0 || K < 0) return TSGU_ERR_SHAPE;
-  if (n_virtual == 0 || nnz_total == 0) return 0;
-  TSGU_DISPATCH_VAL(val_dtype, TSGU_DISPATCH_IDX(idx_dtype, {
-    constexpr int EPVF = 16 / sizeof(V);
-    tsgu::SddmmParams<V, I> p;
-    p.rowptr = (const I*)vrowptr; p.colind = (const I*)colind; p.out_index = (const I*)out_index;
-    p.G = (const V*)G; p.B = (const V*)B; p.out = (V*)out;
-    p.batch = 1; p.n = n_virtual; p.K = K;
-    p.rowptr_bstride = n_virtual; p.nnz_bstride = 0;
-    p.g_bs = 0; p.g_rs = g_rs; p.g_cs = 1; p.b_bs = 0; p.b_rs = b_rs; p.b_cs = 1;
-    p.accumulate = 0; p.row_map = (const I*)row_map;
-    const bool ok = (K % EPVF) == 0 && K / EPVF <= 128 && (b_rs % EPVF) == 0 && (g_rs % EPVF) == 0 && m < 0xffffffffLL &&
-                    b_rs * (int64_t)sizeof(V) < 0xffffffffLL && tsgu::aligned16(B) && tsgu::aligned16(G) &&
-                    tsgu::aligned16(vrowptr) && tsgu::aligned16(colind);
-    if (!ok) return TSGU_ERR_SHAPE;
-    return tsgu::sddmm_tile_dispatch<V, I>(p, nnz_total, tsgu::as_stream(stream));
   }));
   return 0;
 }

@@ -34,12 +34,7 @@ struct SpmmParams {
   int64_t batch, n, K;
   int64_t rowptr_bstride, nnz_bstride;
   int64_t b_bs, b_rs, b_cs, c_bs, ldc;
-  // split-row mode (tile kernel, batch == 1): `rowptr` describes VIRTUAL rows (long rows cut into pieces of
-  // bounded length); row_map[v] >= 0 is the row of C a virtual row is (it was not cut), row_map[v] < 0 says
-  // "piece ~row_map[v] of a cut row": its partial sum goes to `partials` (accumulator type) and
-  // tsgu_sum_row_pieces adds the pieces up in order afterwards.
-  const I* row_map;
-  typename VT<V>::Acc* partials;
+  const I* row_map;  // nullable: CSR row s of item t is row row_map[t*n + s] of C[t] (tsgu_spmm_csr_rowmap)
 };
 
 // EPV: elements per vector load (1 = scalar path that also honours b_cs != 1)
@@ -246,7 +241,7 @@ __global__ void __launch_bounds__(256, TSGU_TILE_MINB(VPL)) spmm_tile_kernel(con
               const char* brow = Bb + (uint64_t)cj * row_bytes;
 #pragma unroll
               for (int w = 0; w < VPL; ++w) {
-                if (EXACT || on[w]) b[u][w] = ldg_gather(reinterpret_cast<const uint4*>(brow + w * (LPR * 16)));
+                if (EXACT || on[w]) b[u][w] = __ldg(reinterpret_cast<const uint4*>(brow + w * (LPR * 16)));
                 else b[u][w] = make_uint4(0, 0, 0, 0);
               }
             }
@@ -271,7 +266,7 @@ __global__ void __launch_bounds__(256, TSGU_TILE_MINB(VPL)) spmm_tile_kernel(con
               const char* brow = Bb + (uint64_t)cj * row_bytes;
 #pragma unroll
               for (int w = 0; w < VPL; ++w) {
-                if (j0 + u < cnt && (EXACT || on[w])) b[u][w] = ldg_gather(reinterpret_cast<const uint4*>(brow + w * (LPR * 16)));
+                if (j0 + u < cnt && (EXACT || on[w])) b[u][w] = __ldg(reinterpret_cast<const uint4*>(brow + w * (LPR * 16)));
                 else b[u][w] = make_uint4(0, 0, 0, 0);
               }
             }
@@ -293,20 +288,10 @@ __global__ void __launch_bounds__(256, TSGU_TILE_MINB(VPL)) spmm_tile_kernel(con
       }
       int64_t dest = c.r0 + lr;
       if (p.row_map) dest = (int64_t)p.row_map[c.item * p.n + dest];
-      if (dest >= 0) {
-        V* Crow = p.C + c.item * p.c_bs + dest * p.ldc;
+      V* Crow = p.C + c.item * p.c_bs + dest * p.ldc;
 #pragma unroll
-        for (int w = 0; w < VPL; ++w)
-          if (EXACT || on[w]) store_vec<V, EPV>(Crow + (int64_t)(w * LPR + gl) * EPV, acc[w]);
-      } else {  // a piece of a cut row: keep the partial in accumulator precision
-        Acc* Prow = p.partials + (~dest) * p.K;
-#pragma unroll
-        for (int w = 0; w < VPL; ++w)
-          if (EXACT || on[w]) {
-#pragma unroll
-            for (int i = 0; i < EPV; ++i) Prow[(int64_t)(w * LPR + gl) * EPV + i] = acc[w][i];
-          }
-      }
+      for (int w = 0; w < VPL; ++w)
+        if (EXACT || on[w]) store_vec<V, EPV>(Crow + (int64_t)(w * LPR + gl) * EPV, acc[w]);
     }
     __syncthreads();  // everyone is done with this stage before it is refilled
   }
@@ -347,22 +332,12 @@ static int spmm_tile_dispatch(const SpmmParams<V, I>& p, int64_t nnz_total, cuda
 #define TSGU_TILE(LPR_, VPL_) \
   return p.perm ? launch_tile<V, I, LPR_, VPL_, true>(p, nnz_total, s) : launch_tile<V, I, LPR_, VPL_, false>(p, nnz_total, s)
   // narrower lane groups with more vectors per lane serve several rows per warp instruction, which
-  // divides the shuffle (col / val broadcast) traffic on the LSU return path (TSGU_LPR_CAP, tile.cuh)
+  // divides the shuffle (col / val broadcast) traffic on the LSU return path (DESIGN.md section 3.1)
   if (kv <= 4) TSGU_TILE(4, 1);
   if (kv <= 8) TSGU_TILE(8, 1);
-#if TSGU_LPR_CAP == 8
   if (kv <= 16) TSGU_TILE(8, 2);
   if (kv <= 32) TSGU_TILE(8, 4);
   if (kv <= 64) TSGU_TILE(16, 4);
-#elif TSGU_LPR_CAP == 16
-  if (kv <= 16) TSGU_TILE(16, 1);
-  if (kv <= 32) TSGU_TILE(16, 2);
-  if (kv <= 64) TSGU_TILE(16, 4);
-#else
-  if (kv <= 16) TSGU_TILE(16, 1);
-  if (kv <= 32) TSGU_TILE(32, 1);
-  if (kv <= 64) TSGU_TILE(32, 2);
-#endif
   TSGU_TILE(32, 4);
 #undef TSGU_TILE
 }
@@ -433,7 +408,7 @@ extern "C" int tsgu_spmm_csr(const void* rowptr, const void* colind, const void*
     p.batch = batch; p.n = n; p.K = K;
     p.rowptr_bstride = rowptr_bstride; p.nnz_bstride = nnz_bstride;
     p.b_bs = b_bs; p.b_rs = b_rs; p.b_cs = b_cs; p.c_bs = c_bs; p.ldc = ldc;
-    p.row_map = nullptr; p.partials = nullptr;
+    p.row_map = nullptr;
     return tsgu::spmm_dispatch<V, I>(p, m, nnz_total, algo, workspace, workspace_bytes, tsgu::as_stream(stream));
   }));
   return 0;
@@ -455,33 +430,8 @@ extern "C" int tsgu_spmm_csr_rowmap(const void* rowptr, const void* colind, cons
     p.batch = batch; p.n = n; p.K = K;
     p.rowptr_bstride = rowptr_bstride; p.nnz_bstride = nnz_bstride;
     p.b_bs = b_bs; p.b_rs = b_rs; p.b_cs = b_cs; p.c_bs = c_bs; p.ldc = ldc;
-    p.row_map = (const I*)row_map; p.partials = nullptr;
+    p.row_map = (const I*)row_map;
     return tsgu::spmm_dispatch<V, I>(p, m, nnz_total, algo, nullptr, 0, tsgu::as_stream(stream));
-  }));
-  return 0;
-}
-
-extern "C" int tsgu_spmm_csr_split(const void* vrowptr, const void* colind, const void* vals, const void* perm,
-                                   const void* row_map, const void* B, void* C, void* partials, int64_t n_virtual,
-                                   int64_t m, int64_t K, int64_t nnz_total, int64_t b_rs, int64_t ldc, int val_dtype,
-                                   int idx_dtype, void* stream) {
-  if (n_virtual < 0 || K < 0) return TSGU_ERR_SHAPE;
-  if (n_virtual == 0 || K == 0) return 0;
-  TSGU_DISPATCH_VAL(val_dtype, TSGU_DISPATCH_IDX(idx_dtype, {
-    constexpr int EPVF = 16 / sizeof(V);
-    tsgu::SpmmParams<V, I> p;
-    p.rowptr = (const I*)vrowptr; p.colind = (const I*)colind; p.vals = (const V*)vals;
-    p.perm = (const I*)perm; p.B = (const V*)B; p.C = (V*)C;
-    p.batch = 1; p.n = n_virtual; p.K = K;
-    p.rowptr_bstride = n_virtual; p.nnz_bstride = 0;
-    p.b_bs = 0; p.b_rs = b_rs; p.b_cs = 1; p.c_bs = 0; p.ldc = ldc;
-    p.row_map = (const I*)row_map; p.partials = (typename tsgu::VT<V>::Acc*)partials;
-    // split-row mode exists only for the persistent-tile kernels: the caller guarantees 128-bit operands
-    const bool ok = (K % EPVF) == 0 && K / EPVF <= 128 && (b_rs % EPVF) == 0 && (ldc % EPVF) == 0 && m < 0xffffffffLL &&
-                    b_rs * (int64_t)sizeof(V) < 0xffffffffLL && tsgu::aligned16(B) && tsgu::aligned16(C) &&
-                    tsgu::aligned16(vrowptr) && tsgu::aligned16(colind) && tsgu::aligned16(vals) && tsgu::aligned16(perm);
-    if (!ok) return TSGU_ERR_SHAPE;
-    return tsgu::spmm_tile_dispatch<V, I>(p, nnz_total, tsgu::as_stream(stream));
   }));
   return 0;
 }

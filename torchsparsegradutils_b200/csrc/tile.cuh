@@ -20,9 +20,6 @@
 #ifndef TSGU_TILE_LOADS
 #define TSGU_TILE_LOADS(VPL) ((VPL) == 1 ? 8 : 16)
 #endif
-#ifndef TSGU_LPR_CAP
-#define TSGU_LPR_CAP 8     // widest lane group the tile kernels use (8 / 16 / 32)
-#endif
 #ifndef TSGU_TILE_STAGE_BYTES
 #define TSGU_TILE_STAGE_BYTES 36864  // colind + vals bytes staged per tile and stage (36 KB: a 224-row tile of a padded
                                      // transpose fits, so a one-item shard runs ONE wave: 0.1319 -> 0.128 ms per step)

@@ -42,9 +42,6 @@
 #ifndef TSGU_WIN_CW
 #define TSGU_WIN_CW 8       // consumer warps per CTA
 #endif
-#ifndef TSGU_WIN_VEC_SLOTS
-#define TSGU_WIN_VEC_SLOTS 0
-#endif
 #ifndef TSGU_WIN_LPR8
 #define TSGU_WIN_LPR8 8     // lanes per row for 8-vector dense rows (8 x 1 vector or 4 x 2 vectors per lane)
 #endif
@@ -212,15 +209,14 @@ __global__ void __launch_bounds__(256) window_plan_kernel(const I* __restrict__ 
 }
 
 // ======================================================================================== kernels
-template <typename V, typename I, int ROWB, bool PERM, bool GROWS = false>
+template <typename V, typename I, int ROWB, bool GROWS = false>
 struct WinStage {
   static constexpr int AI = 16 / (int)sizeof(I), AV = 16 / (int)sizeof(V);
   alignas(128) unsigned char win[TSGU_WIN_ROWS * ROWB];
   alignas(128) unsigned char grows[GROWS ? TSGU_WIN_TMAX * ROWB : 16];  // SDDMM: the tile's rows of the left operand
   alignas(16) I rp[TSGU_WIN_TMAX + 1 + 2 * AI];
   alignas(16) uint16_t lcol[TSGU_WIN_ECAP + 16];
-  alignas(16) V val[PERM ? AV : TSGU_WIN_ECAP + 2 * AV];
-  alignas(16) I prm[PERM ? TSGU_WIN_ECAP + 2 * AI : AI];
+  alignas(16) V val[TSGU_WIN_ECAP + 2 * AV];
 };
 
 #ifndef TSGU_WIN_LOOKAHEAD
@@ -231,9 +227,9 @@ struct WinInfoRing {
   alignas(16) int32_t desc[TSGU_WIN_LOOKAHEAD][WIN_DESC_WORDS];
   alignas(16) I bounds[TSGU_WIN_LOOKAHEAD][2];
 };
-template <typename V, typename I, int ROWB, bool PERM, bool GROWS = false>
+template <typename V, typename I, int ROWB, bool GROWS = false>
 struct WinSmem {
-  WinStage<V, I, ROWB, PERM, GROWS> st[TSGU_WIN_STAGES];
+  WinStage<V, I, ROWB, GROWS> st[TSGU_WIN_STAGES];
   WinInfoRing<I> ring;
   // SpMM with a column-major result: double-buffered CTA scratch for the (rows of one pass) x K transpose; rows are
   // padded by one element (conflict-free column reads).  Sized for 64 rows per pass (4-lane groups).
@@ -247,8 +243,7 @@ struct WinParams {
   const I* rowptr;
   const uint16_t* lcol;
   const int32_t* desc;
-  const V* vals;       // SpMM
-  const I* perm;       // SpMM, nullable
+  const V* vals;       // SpMM, in pattern order
   const I* out_index;  // SDDMM, nullable
   const V* G;          // SDDMM: left dense operand (rows of A)
   const V* B;          // windowed dense operand (columns of A)
@@ -315,8 +310,8 @@ __device__ __forceinline__ void win_fetch_info(const WinParams<V, I>& p, WinInfo
 }
 
 // producer warp: stream a tile into stage `st`
-template <typename V, typename I, int ROWB, bool PERM, bool WITH_VALS>
-__device__ __forceinline__ void win_produce(const WinParams<V, I>& p, WinStage<V, I, ROWB, PERM, !WITH_VALS>& st, uint64_t* bar,
+template <typename V, typename I, int ROWB, bool WITH_VALS>
+__device__ __forceinline__ void win_produce(const WinParams<V, I>& p, WinStage<V, I, ROWB, !WITH_VALS>& st, uint64_t* bar,
                                             const WinTileInfo& ti, int item, int r0, int rows, int lane) {
   using TP = TileProducer<V, I, 0>;
   uint32_t tx = 0;
@@ -337,10 +332,7 @@ __device__ __forceinline__ void win_produce(const WinParams<V, I>& p, WinStage<V
     tx += TP::template span<I>(st.rp, p.rowptr, rp_lo, rp_lo + rows + 1, p.rowptr_len, bar);
     if (ti.e_abs > ti.s_abs) {
       tx += TP::template span<uint16_t>(st.lcol, p.lcol, ti.s_abs, ti.e_abs, p.nnz_len, bar);
-      if constexpr (WITH_VALS) {
-        if constexpr (PERM) tx += TP::template span<I>(st.prm, p.perm, ti.s_abs, ti.e_abs, p.nnz_len, bar);
-        else tx += TP::template span<V>(st.val, p.vals, ti.s_abs, ti.e_abs, p.nnz_len, bar);
-      }
+      if constexpr (WITH_VALS) tx += TP::template span<V>(st.val, p.vals, ti.s_abs, ti.e_abs, p.nnz_len, bar);
     }
   }
   if constexpr (!WITH_VALS) {  // SDDMM: the tile's rows of the upstream gradient (consecutive rows)
@@ -359,8 +351,8 @@ __device__ __forceinline__ void win_produce(const WinParams<V, I>& p, WinStage<V
   if (lane == 0) mbar_expect_tx(bar, tx);  // the only arrival of this phase; also publishes span()'s tail stores
 }
 
-template <typename V, typename I, int ROWB, bool PERM, bool WITH_VALS>
-__device__ __forceinline__ void win_producer_loop(const WinParams<V, I>& p, WinSmem<V, I, ROWB, PERM, !WITH_VALS>& sm, int lane) {
+template <typename V, typename I, int ROWB, bool WITH_VALS>
+__device__ __forceinline__ void win_producer_loop(const WinParams<V, I>& p, WinSmem<V, I, ROWB, !WITH_VALS>& sm, int lane) {
   constexpr int NST = TSGU_WIN_STAGES;
   constexpr int PD = TSGU_WIN_LOOKAHEAD;
   WinInfoRing<I>& ring = sm.ring;
@@ -402,7 +394,7 @@ __device__ __forceinline__ void win_producer_loop(const WinParams<V, I>& p, WinS
     geom(cur, r0, rows);
     const int s = it % NST;
     if (it >= NST) mbar_wait(&sm.empty[s], (uint32_t)((it / NST - 1) & 1));
-    win_produce<V, I, ROWB, PERM, WITH_VALS>(p, sm.st[s], &sm.full[s], ti, cur.item, r0, rows, lane);
+    win_produce<V, I, ROWB, WITH_VALS>(p, sm.st[s], &sm.full[s], ti, cur.item, r0, rows, lane);
     cur.next();
   }
   cp_async_wait<0>();
@@ -410,14 +402,14 @@ __device__ __forceinline__ void win_producer_loop(const WinParams<V, I>& p, WinS
 
 // ------------------------------------------------------------------------------------------ SpMM
 // LPR lanes own a row, VPL 128-bit vectors per lane: LPR * VPL * 16 == ROWB == K * sizeof(V) (exact K only).
-template <typename V, typename I, int LPR, int VPL, int U, bool PERM>
+template <typename V, typename I, int LPR, int VPL, int U>
 __global__ void __launch_bounds__(TSGU_WIN_CW * 32 + 32) spmm_window_kernel(const WinParams<V, I> p) {
   using Acc = typename VT<V>::Acc;
   constexpr int ROWB = LPR * VPL * 16;
   constexpr int EPV = 16 / sizeof(V);
   constexpr int NST = TSGU_WIN_STAGES;
-  using Stage = WinStage<V, I, ROWB, PERM>;
-  using Smem = WinSmem<V, I, ROWB, PERM>;
+  using Stage = WinStage<V, I, ROWB>;
+  using Smem = WinSmem<V, I, ROWB>;
   constexpr int AI = Stage::AI, AV = Stage::AV;
   constexpr int GROUPS = TSGU_WIN_CW * 32 / LPR;
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -434,13 +426,12 @@ __global__ void __launch_bounds__(TSGU_WIN_CW * 32 + 32) spmm_window_kernel(cons
   __syncthreads();
 
   if (warp == TSGU_WIN_CW) {  // ------------------------------------------------ producer warp
-    win_producer_loop<V, I, ROWB, PERM, true>(p, sm, lane);
+    win_producer_loop<V, I, ROWB, true>(p, sm, lane);
     return;
   }
 
   // --------------------------------------------------------------------------- consumer warps
   const int gl = lane % LPR;
-  const unsigned gmask = group_mask<LPR>(lane);
   const int group = tid / LPR;
   const int n32 = (int)p.n;
   WinTileIter ti(blockIdx.x, p.tiles_per_item, (int)gridDim.x);
@@ -459,8 +450,6 @@ __global__ void __launch_bounds__(TSGU_WIN_CW * 32 + 32) spmm_window_kernel(cons
     const int s_al = (int)(((int64_t)s_rel + (int64_t)ti.item * p.nnz_bstride) & 7);
     const uint16_t* slc = st.lcol + s_al - s_rel;                 // slc[rp value] = slot of that entry
     const V* sval = st.val + (s_al & (AV - 1)) - s_rel;
-    const int al4 = s_al - s_rel;  // (e + al4) & 3 == 0  <=>  entry e is 4-aligned in both staged arrays
-    const I* sprm = st.prm + (s_al & (AI - 1)) - s_rel;
 
     for (int lr0 = 0; lr0 < rows; lr0 += GROUPS) {  // warp-uniform trip count; a group past the tile's end idles
       const int lr = lr0 + group;
@@ -485,83 +474,33 @@ __global__ void __launch_bounds__(TSGU_WIN_CW * 32 + 32) spmm_window_kernel(cons
         }
       };
 
-      if constexpr (!PERM) {
-        // A row is walked in chunks of 8, 4, 2, 1 entries: every chunk is full, nothing is predicated.  (Build-time
-        // experiment TSGU_WIN_VEC_SLOTS=1: peel single entries until the staged arrays are 4-entry aligned and read
-        // slots / values as LDS.64 / LDS.128 vectors -- fewer shared-memory wavefronts (95 M -> 77 M on config 3) but
-        // the peel length differs between the rows of a warp, and the divergence costs more: 0.362 -> 0.374 ms.)
-        auto chunk = [&](auto UC, int e) {
-          constexpr int N = decltype(UC)::value;
-          uint32_t slot[N];
-          Acc v[N];
-          if constexpr (TSGU_WIN_VEC_SLOTS && N % 4 == 0) {
+      // A row is walked in chunks of 8, 4, 2, 1 entries: every chunk is full, nothing is predicated.  (Peeling single
+      // entries until the staged arrays are 4-entry aligned and reading slots / values as LDS.64 / LDS.128 vectors
+      // was measured: fewer shared-memory wavefronts (95 M -> 77 M on config 3), but the peel length differs between
+      // the rows of a warp, and the divergence costs more: 0.362 -> 0.374 ms.)
+      auto chunk = [&](auto UC, int e) {
+        constexpr int N = decltype(UC)::value;
+        uint32_t slot[N];
+        Acc v[N];
 #pragma unroll
-            for (int q = 0; q < N / 4; ++q) {
-              const uint2 s4 = *reinterpret_cast<const uint2*>(slc + e + 4 * q);
-              slot[4 * q + 0] = s4.x & 0xffffu; slot[4 * q + 1] = s4.x >> 16;
-              slot[4 * q + 2] = s4.y & 0xffffu; slot[4 * q + 3] = s4.y >> 16;
-              if constexpr (sizeof(V) == 4) {
-                const float4 v4 = *reinterpret_cast<const float4*>(sval + e + 4 * q);
-                v[4 * q + 0] = v4.x; v[4 * q + 1] = v4.y; v[4 * q + 2] = v4.z; v[4 * q + 3] = v4.w;
-              } else {
-                const uint2 v4 = *reinterpret_cast<const uint2*>(sval + e + 4 * q);
-                v[4 * q + 0] = __uint_as_float(v4.x << 16); v[4 * q + 1] = __uint_as_float(v4.x & 0xffff0000u);
-                v[4 * q + 2] = __uint_as_float(v4.y << 16); v[4 * q + 3] = __uint_as_float(v4.y & 0xffff0000u);
-              }
-            }
-          } else {
-#pragma unroll
-            for (int u = 0; u < N; ++u) {
-              slot[u] = slc[e + u];
-              v[u] = VT<V>::to_acc(sval[e + u]);
-            }
-          }
-          uint4 b[N][VPL];
-#pragma unroll
-          for (int u = 0; u < N; ++u)
-#pragma unroll
-            for (int w = 0; w < VPL; ++w) b[u][w] = lds128(win0 + slot[u] * ROWB + w * (LPR * 16));
-#pragma unroll
-          for (int u = 0; u < N; ++u) fma_row(b[u], v[u]);
-        };
-        int e = e0;
-#if TSGU_WIN_VEC_SLOTS
-        while (((e + al4) & 3) && e < e1) { chunk(std::integral_constant<int, 1>{}, e); ++e; }
-#endif
-        if constexpr (U >= 8) for (; e + 8 <= e1; e += 8) chunk(std::integral_constant<int, 8>{}, e);
-        if constexpr (U >= 8) { if (e + 4 <= e1) { chunk(std::integral_constant<int, 4>{}, e); e += 4; } }
-        else for (; e + 4 <= e1; e += 4) chunk(std::integral_constant<int, 4>{}, e);
-        if (e + 2 <= e1) { chunk(std::integral_constant<int, 2>{}, e); e += 2; }
-        if (e < e1) chunk(std::integral_constant<int, 1>{}, e);
-      } else {
-        // values live in the caller's storage order: lanes fetch vals[perm[e]] for a batch of LPR entries
-        // (one 4-byte gather each, issued together), then broadcast them inside the group
-        for (int base = e0; base < e1; base += LPR) {
-          const int el = base + gl;
-          Acc vq = Acc(0);
-          if (el < e1) vq = load_scalar<V>(p.vals + (int64_t)sprm[el]);
-          const int cnt = (e1 - base) < LPR ? (e1 - base) : LPR;
-#pragma unroll
-          for (int j0 = 0; j0 < LPR; j0 += U) {
-            if (j0 < cnt) {
-              uint4 b[U][VPL];
-#pragma unroll
-              for (int u = 0; u < U; ++u) {
-                const bool ok = j0 + u < cnt;
-                const uint32_t slot = ok ? slc[base + j0 + u] : 0u;
-#pragma unroll
-                for (int w = 0; w < VPL; ++w)
-                  b[u][w] = ok ? lds128(win0 + slot * ROWB + w * (LPR * 16)) : make_uint4(0, 0, 0, 0);
-              }
-#pragma unroll
-              for (int u = 0; u < U; ++u) {
-                const Acc vj = shfl_idx(gmask, vq, (j0 + u) % LPR, LPR);  // lanes past the row end hold 0
-                fma_row(b[u], vj);
-              }
-            }
-          }
+        for (int u = 0; u < N; ++u) {
+          slot[u] = slc[e + u];
+          v[u] = VT<V>::to_acc(sval[e + u]);
         }
-      }
+        uint4 b[N][VPL];
+#pragma unroll
+        for (int u = 0; u < N; ++u)
+#pragma unroll
+          for (int w = 0; w < VPL; ++w) b[u][w] = lds128(win0 + slot[u] * ROWB + w * (LPR * 16));
+#pragma unroll
+        for (int u = 0; u < N; ++u) fma_row(b[u], v[u]);
+      };
+      int e = e0;
+      if constexpr (U >= 8) for (; e + 8 <= e1; e += 8) chunk(std::integral_constant<int, 8>{}, e);
+      if constexpr (U >= 8) { if (e + 4 <= e1) { chunk(std::integral_constant<int, 4>{}, e); e += 4; } }
+      else for (; e + 4 <= e1; e += 4) chunk(std::integral_constant<int, 4>{}, e);
+      if (e + 2 <= e1) { chunk(std::integral_constant<int, 2>{}, e); e += 2; }
+      if (e < e1) chunk(std::integral_constant<int, 1>{}, e);
       if (p.c_cs == 1) {  // row-major result: one 128-bit store per vector
         if (active) {
           V* Crow = p.out + (int64_t)ti.item * p.c_bs + (int64_t)(r0 + lr) * p.ldc;
@@ -611,8 +550,8 @@ __global__ void __launch_bounds__(TSGU_WIN_CW * 32 + 32) sddmm_window_kernel(con
   constexpr int NCH = LPR * VPL;  // 16-byte chunks per dense row
   constexpr int EPV = 16 / sizeof(V);
   constexpr int NST = TSGU_WIN_STAGES;
-  using Stage = WinStage<V, I, ROWB, false, true>;
-  using Smem = WinSmem<V, I, ROWB, false, true>;
+  using Stage = WinStage<V, I, ROWB, true>;
+  using Smem = WinSmem<V, I, ROWB, true>;
   constexpr int AI = Stage::AI;
   constexpr int GROUPS = TSGU_WIN_CW * 32 / LPR;
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -629,7 +568,7 @@ __global__ void __launch_bounds__(TSGU_WIN_CW * 32 + 32) sddmm_window_kernel(con
   __syncthreads();
 
   if (warp == TSGU_WIN_CW) {
-    win_producer_loop<V, I, ROWB, false, false>(p, sm, lane);
+    win_producer_loop<V, I, ROWB, false>(p, sm, lane);
     return;
   }
 
@@ -716,17 +655,15 @@ template <typename V, typename I, int LPR, int VPL>
 static int launch_spmm_window(const WinParams<V, I>& p, cudaStream_t s) {
   constexpr int ROWB = LPR * VPL * 16;
   constexpr int U = VPL >= 4 ? 2 : (VPL == 2 ? 4 : 8);
-  static int occ[2] = {0, 0};
-  if (p.perm)
-    return win_launch(spmm_window_kernel<V, I, LPR, VPL, U, true>, (int)sizeof(WinSmem<V, I, ROWB, true>), p.num_tiles, s, &occ[1], p);
-  return win_launch(spmm_window_kernel<V, I, LPR, VPL, U, false>, (int)sizeof(WinSmem<V, I, ROWB, false>), p.num_tiles, s, &occ[0], p);
+  static int occ = 0;
+  return win_launch(spmm_window_kernel<V, I, LPR, VPL, U>, (int)sizeof(WinSmem<V, I, ROWB>), p.num_tiles, s, &occ, p);
 }
 
 template <typename V, typename I, int LPR, int VPL>
 static int launch_sddmm_window(const WinParams<V, I>& p, cudaStream_t s) {
   constexpr int ROWB = LPR * VPL * 16;
   static int occ = 0;
-  return win_launch(sddmm_window_kernel<V, I, LPR, VPL>, (int)sizeof(WinSmem<V, I, ROWB, false, true>), p.num_tiles, s, &occ, p);
+  return win_launch(sddmm_window_kernel<V, I, LPR, VPL>, (int)sizeof(WinSmem<V, I, ROWB, true>), p.num_tiles, s, &occ, p);
 }
 
 template <typename V, typename I>
@@ -779,14 +716,14 @@ extern "C" int tsgu_window_plan(const void* rowptr, const void* colind, int64_t 
 }
 
 template <typename V, typename I>
-static int window_run(bool sddmm, const void* rowptr, const void* lcol, const void* desc, const void* vals, const void* perm,
+static int window_run(bool sddmm, const void* rowptr, const void* lcol, const void* desc, const void* vals,
                       const void* out_index, const void* G, const void* B, void* out, int64_t batch, int64_t n, int64_t K,
                       int64_t rowptr_bstride, int64_t nnz_bstride, int64_t nnz_len, int tile_rows, int64_t g_bs, int64_t g_rs,
                       int64_t b_bs, int64_t b_rs, int64_t c_bs, int64_t ldc, int64_t c_cs, cudaStream_t s) {
   constexpr int EPV = 16 / (int)sizeof(V);
   WinParams<V, I> p;
   p.rowptr = (const I*)rowptr; p.lcol = (const uint16_t*)lcol; p.desc = (const int32_t*)desc;
-  p.vals = (const V*)vals; p.perm = (const I*)perm; p.out_index = (const I*)out_index;
+  p.vals = (const V*)vals; p.out_index = (const I*)out_index;
   p.G = (const V*)G; p.B = (const V*)B; p.out = (V*)out;
   p.batch = batch; p.n = n; p.rowptr_bstride = rowptr_bstride; p.nnz_bstride = nnz_bstride;
   p.rowptr_len = nnz_bstride > 0 ? batch * rowptr_bstride : batch * n + 1;
@@ -796,7 +733,7 @@ static int window_run(bool sddmm, const void* rowptr, const void* lcol, const vo
   p.tiles_per_item = (n + tile_rows - 1) / tile_rows;
   p.num_tiles = p.tiles_per_item * batch;
   const bool ok = (b_rs % EPV) == 0 && (b_bs % EPV) == 0 && aligned16(B) && aligned16(rowptr) && aligned16(lcol) &&
-                  aligned16(vals) && aligned16(perm) &&
+                  aligned16(vals) &&
                   (sddmm ? ((g_rs % EPV) == 0 && (g_bs % EPV) == 0 && aligned16(G))
                          : (c_cs == 1 ? ((ldc % EPV) == 0 && (c_bs % EPV) == 0 && aligned16(out)) : true));
   if (!ok) return TSGU_ERR_SHAPE;
@@ -811,13 +748,13 @@ static int window_run(bool sddmm, const void* rowptr, const void* lcol, const vo
     default: return TSGU_ERR_DTYPE;                                                                                    \
   }
 
-extern "C" int tsgu_spmm_window(const void* rowptr, const void* lcol, const void* desc, const void* vals, const void* perm,
+extern "C" int tsgu_spmm_window(const void* rowptr, const void* lcol, const void* desc, const void* vals,
                                 const void* B, void* C, int64_t batch, int64_t n, int64_t K, int64_t rowptr_bstride,
                                 int64_t nnz_bstride, int64_t nnz_len, int tile_rows, int64_t b_bs, int64_t b_rs, int64_t c_bs,
                                 int64_t ldc, int64_t c_cs, int val_dtype, int idx_dtype, void* stream) {
   if (batch < 0 || n < 0 || K <= 0 || tile_rows < 1 || tile_rows > TSGU_WIN_TMAX) return TSGU_ERR_SHAPE;
   if (batch == 0 || n == 0) return 0;
-  TSGU_WIN_DISPATCH(window_run<V, I>(false, rowptr, lcol, desc, vals, perm, nullptr, nullptr, B, C, batch, n, K, rowptr_bstride,
+  TSGU_WIN_DISPATCH(window_run<V, I>(false, rowptr, lcol, desc, vals, nullptr, nullptr, B, C, batch, n, K, rowptr_bstride,
                                      nnz_bstride, nnz_len, tile_rows, 0, 0, b_bs, b_rs, c_bs, ldc, c_cs, as_stream(stream)));
 }
 
@@ -827,7 +764,7 @@ extern "C" int tsgu_sddmm_window(const void* rowptr, const void* lcol, const voi
                                  int64_t b_rs, int val_dtype, int idx_dtype, void* stream) {
   if (batch < 0 || n < 0 || K <= 0 || tile_rows < 1 || tile_rows > TSGU_WIN_TMAX) return TSGU_ERR_SHAPE;
   if (batch == 0 || n == 0 || nnz_len == 0) return 0;
-  TSGU_WIN_DISPATCH(window_run<V, I>(true, rowptr, lcol, desc, nullptr, nullptr, out_index, G, B, out, batch, n, K,
+  TSGU_WIN_DISPATCH(window_run<V, I>(true, rowptr, lcol, desc, nullptr, out_index, G, B, out, batch, n, K,
                                      rowptr_bstride, nnz_bstride, nnz_len, tile_rows, g_bs, g_rs, b_bs, b_rs, 0, 0, 1,
                                      as_stream(stream)));
 }
