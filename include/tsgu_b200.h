@@ -264,6 +264,51 @@ TSGU_API int tsgu_sddmm_window(const void* rowptr, const void* lcol, const void*
                       int64_t g_bs, int64_t g_rs, int64_t b_bs, int64_t b_rs, int val_dtype, int idx_dtype,
                       void* stream);
 
+/* ------------------------------------------------------------------------------------
+ * Sparse triangular solve  op(A) X = B  (op(A) = A or A^T), level-scheduled and sync-free.
+ *   replaces the torch.triangular_solve / linalg_solve_triangular_compat calls of sparse_solve.py
+ *   SparseTriangularSolve.forward (op(A) x = B) and .backward (op(A)^T gradB = grad), which run
+ *   cuSPARSE's analysis again inside every call; here the analysis is a per-pattern plan.
+ *
+ * The solved matrix is a CSR batch in the conventions above, square (m = n); for op(A) = A^T the
+ * caller passes the CSR of the transposes (tsgu_csr_transpose) and the opposite triangle.  Only
+ * the strictly off-diagonal entries of the requested triangle (`lower`: col < row, else col > row)
+ * and the diagonal are read; entries of the other triangle are ignored, like torch's sparse CSR
+ * triangular_solve.  Rows are addressed flat: row g = t*n + r of item t.
+ *
+ * tsgu_trisolve_levels (once per pattern and triangle): level_out[g] = level of row g - 1
+ *   (int64, 0-based), count_out[g] = number of its off-diagonal dependencies (int64),
+ *   stats_out = uint64[3] {number of levels, total dependencies, status (0 = ok)}; stats_out is
+ *   zeroed on `stream` first.  Sorting the rows stably by level (tsgu_coo_sort on (level, row),
+ *   key_dims = 1) gives `order`, the plan's row order.
+ * tsgu_trisolve_plan: for slot s (row order[s]), with plan_rowptr the exclusive prefix sum of the
+ *   dependency counts in slot order (rows + 1 entries, idx_dtype), writes plan_col (flat row of
+ *   each dependency), plan_pos (position of its value: perm[e] if `perm` is given, else the
+ *   absolute entry position e), and plan_diag[s] (value position of the diagonal entry, -1 if none).
+ * tsgu_trisolve: X (row-major (batch, n, K), contiguous) from B (any strides) over a plan.  `vals`
+ *   is indexed by plan_pos / plan_diag.  unitriangular: the diagonal is taken as 1 (a stored one is
+ *   ignored).  A missing diagonal divides by zero, as the dense solve does.  fp32 and fp64 only
+ *   (TSGU_ERR_DTYPE otherwise).  Results are bit-identical from run to run.
+ * Workspace (tsgu_trisolve_workspace_bytes, both levels and solve): ticket counter, per-row ready
+ *   flags and, as the uint32 at byte offset 8, the status word; each call zeroes it on `stream`.
+ *   Every dependency wait is bounded (about one second): a row whose wait expired is written as NaN
+ *   and the status word (levels: stats_out[2]) becomes non-zero, so the kernels always terminate.
+ * ---------------------------------------------------------------------------------- */
+TSGU_API size_t tsgu_trisolve_workspace_bytes(int64_t batch, int64_t n);
+TSGU_API int tsgu_trisolve_levels(const void* rowptr, const void* colind, int64_t batch, int64_t n,
+                         int64_t rowptr_bstride, int64_t nnz_bstride, int idx_dtype, int lower,
+                         void* level_out, void* count_out, void* stats_out, void* workspace,
+                         size_t workspace_bytes, void* stream);
+TSGU_API int tsgu_trisolve_plan(const void* rowptr, const void* colind, const void* perm, int64_t batch, int64_t n,
+                       int64_t rowptr_bstride, int64_t nnz_bstride, int idx_dtype, int lower,
+                       const void* order, const void* plan_rowptr, void* plan_col, void* plan_pos,
+                       void* plan_diag, void* stream);
+TSGU_API int tsgu_trisolve(const void* plan_rowptr, const void* plan_col, const void* plan_pos,
+                  const void* plan_diag, const void* order, const void* vals, const void* B, void* X,
+                  int64_t batch, int64_t n, int64_t K, int64_t b_bs, int64_t b_rs, int64_t b_cs,
+                  int unitriangular, int val_dtype, int idx_dtype, void* workspace, size_t workspace_bytes,
+                  void* stream);
+
 #ifdef __cplusplus
 }
 #endif

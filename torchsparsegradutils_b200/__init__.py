@@ -14,6 +14,7 @@ from .rsample import rsample_transform
 from .encoders import PairwiseValueAssembler
 from .sddmm import block_diag_operand, lstsq_grad_A, sddmm, solve_grad_A
 from .sparse_matmul import SparseMatMul, sparse_mm
+from .triangular_solve import SparseTriangularSolve, sparse_triangular_solve
 
-__all__ = ["sparse_mm", "SparseMatMul", "sddmm", "solve_grad_A", "lstsq_grad_A", "block_diag_operand", "PairwiseValueAssembler", "batch_sparse_mv", "rsample_transform", "GraphedSparseMM", "utils", "clear_pattern_cache", "prepare_pattern", "set_pattern_cache_capacity"]
+__all__ = ["sparse_mm", "SparseMatMul", "sparse_triangular_solve", "SparseTriangularSolve", "sddmm", "solve_grad_A", "lstsq_grad_A", "block_diag_operand", "PairwiseValueAssembler", "batch_sparse_mv", "rsample_transform", "GraphedSparseMM", "utils", "clear_pattern_cache", "prepare_pattern", "set_pattern_cache_capacity"]
 __version__ = "0.1.0"

@@ -60,6 +60,10 @@ _SIGNATURES = {
     "tsgu_window_plan": (_I, [_P, _P, _L, _L, _L, _L, _I, _I, _P, _P, _P, _P]),
     "tsgu_spmm_window": (_I, [_P, _P, _P, _P, _P, _P, _L, _L, _L, _L, _L, _L, _I, _L, _L, _L, _L, _L, _I, _I, _P]),
     "tsgu_sddmm_window": (_I, [_P, _P, _P, _P, _P, _P, _P, _L, _L, _L, _L, _L, _L, _I, _L, _L, _L, _L, _I, _I, _P]),
+    "tsgu_trisolve_workspace_bytes": (_Z, [_L, _L]),
+    "tsgu_trisolve_levels": (_I, [_P, _P, _L, _L, _L, _L, _I, _I, _P, _P, _P, _P, _Z, _P]),
+    "tsgu_trisolve_plan": (_I, [_P, _P, _P, _L, _L, _L, _L, _I, _I, _P, _P, _P, _P, _P, _P]),
+    "tsgu_trisolve": (_I, [_P, _P, _P, _P, _P, _P, _P, _P, _L, _L, _L, _L, _L, _L, _I, _I, _I, _P, _Z, _P]),
 }
 EXPORTED_SYMBOLS = tuple(_SIGNATURES)
 

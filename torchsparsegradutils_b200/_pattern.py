@@ -87,6 +87,8 @@ def pattern_nbytes(p) -> int:
     for extra in p.extras.values():
         if isinstance(extra, WindowPlan):
             extra = (extra.lcol, extra.desc)
+        elif isinstance(extra, TriPlan):
+            extra = (extra.order, extra.rowptr, extra.col, extra.pos, extra.diag)
         total += sum(_tensor_bytes(t) for t in (extra if isinstance(extra, (tuple, list)) else (extra,)))
     return total + pattern_nbytes(p._transpose)
 
@@ -353,6 +355,22 @@ def window_plan(p: "CsrPattern") -> Optional[WindowPlan]:
                 plan = WindowPlan(launched[0], launched[1], launched[3], max_w, max_runs, max_entries)
     p.extras["window"] = plan
     return plan
+
+
+# ------------------------------------------------------------------------------ triangular-solve plans
+@dataclass
+class TriPlan:
+    """Per-pattern plan of the level-scheduled triangular solve (csrc/trisolve.cu), one per solved triangle and
+    transpose flag: rows in level order and, per slot, the dependencies (flat row, value position) and the diagonal's
+    value position (-1: none).  Kept in ``CsrPattern.extras``."""
+
+    order: torch.Tensor   # (rows,) flat row of each slot
+    rowptr: torch.Tensor  # (rows + 1,) dependency offsets per slot
+    col: torch.Tensor     # (deps,) flat row of each dependency
+    pos: torch.Tensor     # (deps,) position of its value in the value array the solve reads
+    diag: torch.Tensor    # (rows,) position of the diagonal value, -1 if none
+    levels: int
+    idx: int
 
 
 def _build_transpose(p: CsrPattern) -> CsrPattern:
@@ -641,23 +659,50 @@ def coo_pattern(A: torch.Tensor) -> CooPattern:
             csr = _coo_to_flat_csr(ind, batch, n, m, None, idx, keep=(ind,))
             pat = CooPattern(csr, None, ind, None, None, nnz)
         else:
-            perm, srt = _sort_coo(ind, dims, 3, idx, True)
-            dup = False
-            if nnz > 1:
-                first = torch.ones(nnz, dtype=torch.bool, device=ind.device)
-                first[1:] = (srt[:, 1:] != srt[:, :-1]).any(dim=0)
-                dup = not nat.host_read(first.all())[0]  # one-off host sync per pattern (sizes the gradient)
-            if not dup:
-                csr = _coo_to_flat_csr(ind, batch, n, m, perm, idx, keep=(ind,))
-                pat = CooPattern(csr, None, srt, None, perm, nnz)
-            else:
-                # the reference coalesces every item before multiplying (utils/utils.py:580), so both
-                # the product and the gradient live on the sorted unique pattern
-                uniq = srt[:, first].contiguous()
-                starts = torch.nonzero(first).flatten()
-                seg = torch.cat([starts, starts.new_tensor([nnz])]).to(nat.IDX_TORCH[idx])
-                csr = _coo_to_flat_csr(uniq, batch, n, m, None, idx, keep=(ind,))
-                pat = CooPattern(csr, None, uniq, seg, perm, uniq.shape[1])
+            pat = _coo_unique(ind, dims, batch, n, m, idx)
+    pat.cache_key = key
+    _cache_put(key, pat, (ind_key,))
+    return pat
+
+
+def _coo_unique(ind: torch.Tensor, dims, batch: int, n: int, m: int, idx: int) -> CooPattern:
+    """Full lexicographic sort of uncoalesced coordinates; duplicates, if any, are coalesced onto the sorted unique
+    pattern (seg / sort_perm sum their values), otherwise the CSR reads values through the sort permutation."""
+    nnz = ind.shape[1]
+    perm, srt = _sort_coo(ind, dims, len(dims), idx, True)
+    dup = False
+    if nnz > 1:
+        first = torch.ones(nnz, dtype=torch.bool, device=ind.device)
+        first[1:] = (srt[:, 1:] != srt[:, :-1]).any(dim=0)
+        dup = not nat.host_read(first.all())[0]  # one-off host sync per pattern (sizes the gradient)
+    if not dup:
+        csr = _coo_to_flat_csr(ind, batch, n, m, perm, idx, keep=(ind,))
+        return CooPattern(csr, None, srt, None, perm, nnz)
+    # the reference coalesces every item before multiplying (utils/utils.py:580), so both
+    # the product and the gradient live on the sorted unique pattern
+    uniq = srt[:, first].contiguous()
+    starts = torch.nonzero(first).flatten()
+    seg = torch.cat([starts, starts.new_tensor([nnz])]).to(nat.IDX_TORCH[idx])
+    csr = _coo_to_flat_csr(uniq, batch, n, m, None, idx, keep=(ind,))
+    return CooPattern(csr, None, uniq, seg, perm, uniq.shape[1])
+
+
+def coo_unique_pattern(A: torch.Tensor) -> CooPattern:
+    """Pattern of a COO tensor with duplicates coalesced, also for 2-D input (``coo_pattern`` keeps the duplicates of
+    an uncoalesced 2-D tensor as separate entries, which a product may, but a triangular solve may not: its diagonal
+    must be one value).  Same cache as ``coo_pattern``."""
+    if A.dim() == 3 or A.is_coalesced():
+        return coo_pattern(A)
+    ind = A._indices()
+    key = ("coo-unique", _index_key(ind), tuple(A.shape), ind.device)
+    hit = _cache_get(key, (ind,))
+    if hit is not None:
+        return hit
+    ind_key = ind
+    if ind.stride(1) != 1:
+        ind = ind.contiguous()
+    n, m = A.shape
+    pat = _coo_unique(ind, (n, m), 1, n, m, _internal_idx(1, n, m, ind.shape[1]))
     pat.cache_key = key
     _cache_put(key, pat, (ind_key,))
     return pat

@@ -13,7 +13,7 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-SOURCES = ["api.cu", "spmm.cu", "sddmm.cu", "index.cu", "merge.cu", "window.cu"]
+SOURCES = ["api.cu", "spmm.cu", "sddmm.cu", "index.cu", "merge.cu", "window.cu", "trisolve.cu"]
 HEADERS = ["common.cuh", "tile.cuh", os.path.join(ROOT, "include", "tsgu_b200.h")]
 LIB = os.path.join(os.path.dirname(HERE), "libtsgu_b200.so")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")

@@ -9,7 +9,8 @@ The reference runs ``_batch_sparse_mv(spmm, L, eta)`` -- ``sparse_mm`` on a tran
 result is transposed / permuted back -- followed by two elementwise adds (``+ eta`` at ``:362``, ``loc +`` at ``:389``)
 on strided views.  Here the product is the same ``sparse_mm`` call and everything after it is ONE pass
 (``tsgu_pack_dense_add``): the layout change back to eps's layout, ``+ eta`` and ``+ loc`` in a single coalesced kernel.
-The precision (``precision_tril``) parameterisations need a triangular solve and stay out of scope.
+The precision (``precision_tril``) parameterisations need a triangular solve (``sparse_triangular_solve``); their
+``rsample`` / ``log_prob`` are not built here yet.
 """
 from __future__ import annotations
 

@@ -77,6 +77,44 @@ def stencil27_csr(D, dtype=torch.float32, index_dtype=torch.int32, device="cuda"
     return torch.sparse_csr_tensor(crow.to(index_dtype), col.to(index_dtype), vals, (n, n))
 
 
+def random_lower_csr(batch, n, per_row, dtype=torch.float32, index_dtype=torch.int32, device="cuda", seed=6):
+    """Random lower triangle: row r holds min(r, per_row - 1) distinct uniform columns below the diagonal plus the
+    diagonal (sorted).  Every item has the same row lengths, so a batch is a valid batched CSR.  batch=None -> 2-D.
+    Values from :func:`triangular_values`."""
+    g = _gen(device, seed)
+    b, k = batch or 1, per_row - 1
+    r = torch.arange(n, device=device)
+    span = (r - k + 1).clamp(min=1)  # draws in [0, r - k]: sorted + arange(k) gives k distinct columns below r
+    x = (torch.rand((b, n, k), generator=g, device=device) * span[None, :, None]).long().sort(dim=2).values
+    x = x + torch.arange(k, device=device)
+    cols = torch.cat([x, r.expand(b, n).unsqueeze(-1)], dim=2)
+    keep = torch.cat([torch.arange(k, device=device)[None, :] < r.clamp(max=k)[:, None],
+                      torch.ones(n, 1, dtype=torch.bool, device=device)], dim=1)  # rows r < k: columns 0..r-1
+    col = cols[keep.expand(b, n, k + 1)].reshape(b, -1)
+    crow = torch.zeros(n + 1, dtype=torch.int64, device=device)
+    crow[1:] = keep.sum(dim=1).cumsum(0)
+    crow = crow.repeat(b, 1)
+    if batch is None:
+        crow, col = crow[0], col[0]
+    shape = (batch, n, n) if batch is not None else (n, n)
+    A = torch.sparse_csr_tensor(crow.to(index_dtype), col.to(index_dtype), torch.zeros(col.shape, device=device), shape)
+    return triangular_values(A, dtype, seed=seed + 1)
+
+
+def triangular_values(A, dtype=torch.float32, seed=7):
+    """A's CSR pattern with well-conditioned triangular-solve values: off-diagonal entries U(0,1) / row length,
+    diagonal entries U(1,2)."""
+    crow, col = A.crow_indices(), A.col_indices()
+    n = A.shape[-1]
+    crow2, col2 = crow.reshape(-1, n + 1).long(), col.reshape(crow.numel() // (n + 1), -1).long()
+    lens = crow2.diff(dim=1)
+    row = torch.repeat_interleave(torch.arange(n, device=col.device).repeat(crow2.shape[0]), lens.reshape(-1),
+                                  output_size=col2.numel()).reshape(col2.shape)
+    u = torch.rand(col2.shape, generator=_gen(col.device, seed), device=col.device, dtype=torch.float64)
+    vals = torch.where(col2 == row, 1.0 + u, u / lens.gather(1, row).clamp(min=1)).to(dtype).reshape(col.shape)
+    return torch.sparse_csr_tensor(crow, col, vals, A.shape)
+
+
 def rmat_csr(scale, edge_factor=16, dtype=torch.bfloat16, index_dtype=torch.int32, device="cuda", seed=4,
              a=0.57, b=0.19, c=0.19):
     """Config 4: Graph500 R-MAT (a,b,c,d = .57,.19,.19,.05), 2^scale vertices, edge_factor*2^scale draws,
