@@ -188,6 +188,27 @@ def test_uniform_rows_gate_of_k_slicing():
     assert not pat(torch.zeros(7, dtype=torch.int32), 1, 6, 6, 0).uniform_rows
 
 
+def test_kernel_family_choice(monkeypatch):
+    """`choose_algo`: merge-path only for a single matrix whose longest row exceeds both 256 entries and 16 x the mean;
+    TSGU_B200_ALGO forces a family, read when a pattern is built (not at import)."""
+    from torchsparsegradutils_b200 import _native as nat
+    from torchsparsegradutils_b200._pattern import choose_algo
+
+    monkeypatch.delenv("TSGU_B200_ALGO", raising=False)
+    assert choose_algo(257, 1, 100, 1000) == nat.ALGO_MERGE  # 257 > 256 and > 16 x 10
+    assert choose_algo(256, 1, 100, 1000) == nat.ALGO_AUTO  # not above 256 entries
+    assert choose_algo(400, 1, 100, 3000) == nat.ALGO_AUTO  # 400 < 16 x 30
+    assert choose_algo(481, 1, 100, 3000) == nat.ALGO_MERGE  # 481 > 16 x 30
+    assert choose_algo(480, 1, 100, 3000) == nat.ALGO_AUTO
+    assert choose_algo(10**6, 4, 100, 1000) == nat.ALGO_AUTO  # a batch always takes the row-tile kernels
+    assert choose_algo(None, 4, 100, 1000) == nat.ALGO_AUTO
+    assert choose_algo(0, 1, 100, 0) == nat.ALGO_AUTO and choose_algo(None, 1, 0, 0) == nat.ALGO_AUTO  # empty
+    monkeypatch.setenv("TSGU_B200_ALGO", "merge")
+    assert choose_algo(1, 1, 100, 100) == nat.ALGO_MERGE and choose_algo(None, 4, 0, 0) == nat.ALGO_MERGE
+    monkeypatch.setenv("TSGU_B200_ALGO", "RowSplit")
+    assert choose_algo(10**6, 1, 100, 1000) == nat.ALGO_ROWSPLIT
+
+
 def test_pattern_checksum_schedule_and_host_fingerprint(monkeypatch):
     """Which cache hits re-check a pattern's index checksum (default 1, 2, 4, 8, ...; "1" all; "0" none), the host
     restatement of tsgu_fingerprint (position-weighted sum: order of equal values matters), and the longest-row rule

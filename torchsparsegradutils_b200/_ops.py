@@ -2,12 +2,14 @@
 from __future__ import annotations
 
 import os
-from typing import Optional
+from typing import TYPE_CHECKING, Optional
 
 import torch
 
 from . import _native as nat
-from ._pattern import CsrPattern, WindowPlan, window_plan
+
+if TYPE_CHECKING:
+    from ._pattern import CsrPattern, WindowPlan
 
 _VEC_ELEMS = {torch.float32: 4, torch.float64: 2, torch.bfloat16: 8}
 _PREGATHER_MIN_NNZ = 1 << 18
@@ -196,7 +198,7 @@ def _window_for(pat: CsrPattern, algo: int, *dense: torch.Tensor) -> Optional[Wi
         return None
     if not all(_vector_ready(x) for x in dense):
         return None
-    return window_plan(pat)
+    return pat.window
 
 
 def _spmm_window(pat: CsrPattern, wp: WindowPlan, vals: torch.Tensor, dense: torch.Tensor, tag: str,

@@ -33,6 +33,7 @@ from typing import Optional
 import torch
 
 from . import _native as nat
+from . import _ops
 
 _CACHE_CAPACITY = 16
 _CACHE_BYTES = int(os.environ.get("TSGU_B200_PATTERN_CACHE_BYTES", str(8 << 30)))  # derived structures + kept index tensors
@@ -84,10 +85,10 @@ def pattern_nbytes(p) -> int:
                 + (_tensor_bytes(p.out_index) if p.out_index is not p.csr.perm else 0))
     total = sum(_tensor_bytes(t) for t in (p.rowptr, p.colind, p.perm))
     total += sum(_tensor_bytes(t) for t in p.keep if isinstance(t, torch.Tensor) and t is not p.rowptr and t is not p.colind)
+    if p.window is not None:
+        total += _tensor_bytes(p.window.lcol) + _tensor_bytes(p.window.desc)
     for extra in p.extras.values():
-        if isinstance(extra, WindowPlan):
-            extra = (extra.lcol, extra.desc)
-        elif isinstance(extra, TriPlan):
+        if isinstance(extra, TriPlan):
             extra = (extra.order, extra.rowptr, extra.col, extra.pos, extra.diag)
         total += sum(_tensor_bytes(t) for t in (extra if isinstance(extra, (tuple, list)) else (extra,)))
     return total + pattern_nbytes(p._transpose)
@@ -155,13 +156,29 @@ class CsrPattern:
     keep: tuple = ()  # tensors whose storage must outlive this pattern (cache-key owners)
     row_map: Optional[torch.Tensor] = None  # rows were permuted: CSR row s of item t is output row row_map[t*n + s]
     padded: bool = False  # perm holds -1 entries (explicit zeros): the values MUST go through gather_values, never the in-kernel perm path
-    extras: dict = field(default_factory=dict, repr=False)  # per-pattern plans built lazily by _ops (window plans, ...)
+    window: Optional["WindowPlan"] = field(default=None, repr=False)  # column-window plan, decided when the pattern is built
+    extras: dict = field(default_factory=dict, repr=False)  # per-pattern plans built lazily (triangular-solve plans, ...)
     fingerprint: Optional[torch.Tensor] = field(default=None, repr=False)
     cache_key: Optional[tuple] = field(default=None, repr=False)
     _transpose: Optional["CsrPattern"] = field(default=None, repr=False)
     _transpose_uses: int = field(default=0, repr=False)
     _uniform: Optional[bool] = field(default=None, repr=False)
     _lock: threading.Lock = field(default_factory=threading.Lock, repr=False)
+
+    # operand view of a CSR tensor's pattern (see pattern_of): values in storage order, gradient on A's own crow/col
+    out_index = None
+    grad_indices = None
+
+    @property
+    def csr(self) -> "CsrPattern":
+        return self
+
+    @property
+    def nnz_out(self) -> int:
+        return self.nnz_total
+
+    def values(self, A: torch.Tensor) -> torch.Tensor:
+        return aligned_contiguous(A.values())
 
     @property
     def device(self) -> torch.device:
@@ -209,46 +226,36 @@ class CsrPattern:
 _ALGO_ENV = {"auto": None, "rowsplit": nat.ALGO_ROWSPLIT, "merge": nat.ALGO_MERGE}
 
 
-def choose_algo(rowptr: torch.Tensor, batch: int, n: int, nnz_total: int) -> int:
-    """Row-split (regular rows) or merge-path (skewed rows) -- decided once per pattern.
+def choose_algo(max_row: Optional[int], batch: int, n: int, nnz_total: int) -> int:
+    """Row-split (regular rows) or merge-path (skewed rows) -- decided once per pattern from its longest row (None: not
+    read, as for a batch of matrices, which always takes the row-tile kernels).
 
     Merge-path pays a fix-up pass and per-entry row bookkeeping, so it is only picked when one row
     is both long in absolute terms (> 256 entries: it would keep one lane group busy for dozens of gather batches
     while the rest of its tile idles) and far above the mean (> 16 x).  Power-law graphs qualify, and so does every
     row block of one: the tail rows of an R-MAT matrix handed to a rank by row sharding still hold rows of several
     hundred entries among rows of 8 (with the round-1 thresholds, 1024 / 32 x, that shard fell to the row-tile
-    kernels and its rank took 25 ms per step).  One host sync per new pattern.  ``TSGU_B200_ALGO=auto|rowsplit|merge`` overrides the heuristic (benchmarking only).
+    kernels and its rank took 25 ms per step).  ``TSGU_B200_ALGO=auto|rowsplit|merge`` overrides the heuristic
+    (benchmarking only).
     """
     forced = _ALGO_ENV.get(os.environ.get("TSGU_B200_ALGO", "auto").lower())
     if forced is not None:
         return forced
-    if batch != 1 or nnz_total == 0 or n == 0:
+    if max_row is None or batch != 1 or nnz_total == 0 or n == 0:
         return nat.ALGO_AUTO
-    flat = rowptr.reshape(-1)  # batch == 1: torch batched CSR keeps a leading dim of 1
-    return _algo_from_max_row(nat.host_read((flat[1:] - flat[:-1]).max())[0], n, nnz_total)
-
-
-def _algo_from_max_row(max_row: int, n: int, nnz_total: int) -> int:
     return nat.ALGO_MERGE if (max_row > 256 and max_row > 16 * (nnz_total / n)) else nat.ALGO_AUTO
 
 
-def _needs_row_stats(batch: int, n: int, nnz_total: int) -> bool:
-    """Does choose_algo need the longest row (a device reduction + host read) for this pattern?"""
-    forced = _ALGO_ENV.get(os.environ.get("TSGU_B200_ALGO", "auto").lower())
-    return forced is None and batch == 1 and nnz_total > 0 and n > 0
-
-
-def _analyse(rowptr: torch.Tensor, colind: torch.Tensor, batch: int, n: int, m: int, rowptr_bstride: int, nnz_bstride: int,
-             nnz_total: int, idx: int, extra=None):
-    """Everything the host must know about a new pattern, gathered with ONE host read: the longest row (kernel family),
-    the verdict of a speculatively launched column-window plan, and optional extra device scalars of the caller.
-    Returns (algo, WindowPlan | None, extra values, longest row | None)."""
-    parts = []
-    want_rows = _needs_row_stats(batch, n, nnz_total)
+def _new_pattern(rowptr: torch.Tensor, colind: torch.Tensor, perm: Optional[torch.Tensor], batch: int, n: int, m: int,
+                 rowptr_bstride: int, nnz_bstride: int, nnz_total: int, idx: int, keep=(), extra=None):
+    """The CsrPattern of a new structure, with everything the host must know about it gathered in ONE host read: the
+    longest row (kernel family, uniform_rows), the verdict of a speculatively launched column-window plan, and optional
+    extra device scalars of the caller.  Returns (pattern, host values of `extra`)."""
     launched = _window_plan_launch(rowptr, colind, batch, n, m, rowptr_bstride, nnz_bstride, nnz_total, idx)
-    # the longest row rides along whenever something is read anyway (it also answers CsrPattern.uniform_rows, which would
-    # otherwise cost the first forward a host sync of its own)
-    with_rows = nnz_total > 0 and n > 0 and (want_rows or launched is not None or extra is not None)
+    # the longest row picks the kernel family of a single matrix, and rides along whenever something is read anyway (it
+    # also answers CsrPattern.uniform_rows, which would otherwise cost the first forward a host sync of its own)
+    with_rows = nnz_total > 0 and n > 0 and (batch == 1 or launched is not None or extra is not None)
+    parts = []
     if with_rows:
         flat = rowptr.reshape(-1)  # differences across item boundaries of a (b, n+1) rowptr are <= 0: harmless for a max
         parts.append((flat[1:] - flat[:-1]).max().reshape(1).long())
@@ -257,22 +264,19 @@ def _analyse(rowptr: torch.Tensor, colind: torch.Tensor, batch: int, n: int, m: 
     if extra is not None:
         parts.append(extra.reshape(-1).long())
     host = nat.host_read(torch.cat(parts)) if parts else []  # the one host sync
-    pos = 0
-    max_row = None
-    if with_rows:
-        max_row = host[0]
-        pos = 1
-    if want_rows:
-        algo = _algo_from_max_row(max_row, n, nnz_total)
-    else:
-        algo = choose_algo(rowptr, batch, n, nnz_total)  # forced / batched / empty: no device read
-    plan = None
+    max_row = host[0] if with_rows else None
+    pos = 1 if with_rows else 0
+    algo = choose_algo(max_row, batch, n, nnz_total)
+    window = None
     if launched is not None:
         failed, max_w, max_runs, max_entries = host[pos:pos + 4]
         pos += 4
         if failed == 0 and algo == nat.ALGO_AUTO:
-            plan = WindowPlan(launched[0], launched[1], launched[3], max_w, max_runs, max_entries)
-    return algo, plan, host[pos:], max_row
+            window = WindowPlan(launched[0], launched[1], launched[3], max_w, max_runs, max_entries)
+    pat = CsrPattern(rowptr, colind, perm, batch, n, m, rowptr_bstride, nnz_bstride, nnz_total, idx, algo=algo, keep=keep,
+                     window=window)
+    pat._uniform = _uniform_from(max_row, batch * n, nnz_total)
+    return pat, host[pos:]
 
 
 def _uniform_from(max_row: Optional[int], rows: int, nnz_total: int) -> Optional[bool]:
@@ -341,20 +345,9 @@ def _window_plan_launch(rowptr, colind, batch, n, m, rowptr_bstride, nnz_bstride
 
 def window_plan(p: "CsrPattern") -> Optional[WindowPlan]:
     """Column-window plan of a pattern, or None when the pattern is not structured enough (some tile of consecutive
-    rows touches more distinct columns / runs than a shared-memory window holds).  Normally decided together with the
-    kernel family when the pattern is created (`_analyse`: one host read for both); built here on demand otherwise."""
-    if "window" in p.extras:
-        return p.extras["window"]
-    plan = None
-    if p.algo == nat.ALGO_AUTO:
-        launched = _window_plan_launch(p.rowptr, p.colind, p.batch, p.n, p.m, p.rowptr_bstride, p.nnz_bstride, p.nnz_total,
-                                       p.idx)
-        if launched is not None:
-            failed, max_w, max_runs, max_entries = nat.host_read(launched[2])
-            if failed == 0:
-                plan = WindowPlan(launched[0], launched[1], launched[3], max_w, max_runs, max_entries)
-    p.extras["window"] = plan
-    return plan
+    rows touches more distinct columns / runs than a shared-memory window holds).  Decided together with the kernel
+    family when the pattern is built (`_new_pattern`: one host read for both)."""
+    return p.window
 
 
 # ------------------------------------------------------------------------------ triangular-solve plans
@@ -373,33 +366,35 @@ class TriPlan:
     idx: int
 
 
-def _build_transpose(p: CsrPattern) -> CsrPattern:
+def _transpose_csr(p: CsrPattern):
+    """Plain CSR of the transposes of `p` (flat over batch*m rows, stable, no length sorting or padding) from
+    tsgu_csr_transpose, its perm composed to point into p's value storage.  Returns (rowptr, colind, perm, idx)."""
     dev = p.device
-    out_idx = _internal_idx(p.batch, p.m, p.n, p.nnz_total)
-    odt = nat.IDX_TORCH[out_idx]
-    rowptrT = torch.empty(p.batch * p.m + 1, dtype=odt, device=dev)
-    colindT = torch.empty(p.nnz_total, dtype=odt, device=dev)
-    permT = torch.empty(p.nnz_total, dtype=odt, device=dev)
+    idx = _internal_idx(p.batch, p.m, p.n, p.nnz_total)
+    odt = nat.IDX_TORCH[idx]
+    rowptr = torch.empty(p.batch * p.m + 1, dtype=odt, device=dev)
+    colind = torch.empty(p.nnz_total, dtype=odt, device=dev)
+    perm = torch.empty(p.nnz_total, dtype=odt, device=dev)
     L = nat.lib()
     with torch.cuda.device(dev):
-        ws_bytes = L.tsgu_csr_transpose_workspace_bytes(p.batch, p.m, p.nnz_total, out_idx)
-        ws = nat.workspace(ws_bytes, dev)
+        ws = nat.workspace(L.tsgu_csr_transpose_workspace_bytes(p.batch, p.m, p.nnz_total, idx), dev)
         nat.check(L.tsgu_csr_transpose(nat.ptr(p.rowptr), nat.ptr(p.colind), p.batch, p.n, p.m, p.rowptr_bstride,
-                                       p.nnz_bstride, p.nnz_total, p.idx, nat.ptr(rowptrT), nat.ptr(colindT),
-                                       nat.ptr(permT), out_idx, nat.ptr(ws), ws.numel(), nat.stream_ptr(dev)),
+                                       p.nnz_bstride, p.nnz_total, p.idx, nat.ptr(rowptr), nat.ptr(colind),
+                                       nat.ptr(perm), idx, nat.ptr(ws), ws.numel(), nat.stream_ptr(dev)),
                   "tsgu_csr_transpose")
     if p.perm is not None and p.nnz_total > 0:
         # entries of p are themselves a permutation of the caller's value storage: compose once
-        permT = p.perm.to(odt).index_select(0, permT.long()) if p.perm.dtype != odt else p.perm.index_select(0, permT.long())
-    nnzT = p.nnz_total
+        perm = p.perm.to(odt).index_select(0, perm.long())
+    return rowptr, colind, perm, idx
+
+
+def _build_transpose(p: CsrPattern) -> CsrPattern:
+    rowptrT, colindT, permT, out_idx = _transpose_csr(p)
     lensT = (rowptrT[1:] - rowptrT[:-1]).long()
     padded_total = ((lensT + (_ROW_PAD - 1)) // _ROW_PAD * _ROW_PAD).sum()  # device scalar, read with the other verdicts
-    algo, plan, (padded_total,), max_row = _analyse(rowptrT, colindT, p.batch, p.m, p.n, p.m, 0, nnzT, out_idx,
-                                                    extra=padded_total)
-    patT = CsrPattern(rowptrT, colindT, permT, p.batch, p.m, p.n, p.m, 0, nnzT, out_idx, algo=algo)
-    patT._uniform = _uniform_from(max_row, p.batch * p.m, nnzT)
-    patT.extras["window"] = plan
-    if algo == nat.ALGO_AUTO and nnzT >= _PAD_MIN_NNZ and plan is None:
+    patT, (padded_total,) = _new_pattern(rowptrT, colindT, permT, p.batch, p.m, p.n, p.m, 0, p.nnz_total, out_idx,
+                                         extra=padded_total)
+    if patT.algo == nat.ALGO_AUTO and patT.nnz_total >= _PAD_MIN_NNZ and patT.window is None:
         # no column-window structure: the row-tile kernels take it, and two layout optimisations of a structure WE own
         # apply -- later, if the pattern turns out to be reused (CsrPattern.transpose).  No further host sync then: the
         # padded size came with the verdicts above.
@@ -425,7 +420,6 @@ def _optimise_layout(patT: CsrPattern) -> CsrPattern:
         rowptrT, colindT, permT = _pad_rows(rowptrT, colindT, permT, _ROW_PAD, padded_total)
     new = CsrPattern(rowptrT, colindT, permT, patT.batch, patT.n, patT.m, patT.n, 0, permT.numel(), patT.idx,
                      algo=patT.algo, row_map=row_map, padded=permT.numel() > patT.nnz_total)
-    new.extras["window"] = None
     new._uniform = patT._uniform
     return new
 
@@ -566,11 +560,7 @@ def csr_pattern(A: torch.Tensor) -> CsrPattern:
     crow_c, col_c = aligned_contiguous(crow), aligned_contiguous(col)
     nnz_item = col_c.shape[-1]
     idx = nat.idx_enum(crow.dtype)
-    algo, plan, _, max_row = _analyse(crow_c, col_c, batch, n, m, n + 1, nnz_item, batch * nnz_item, idx)
-    pat = CsrPattern(crow_c, col_c, None, batch, n, m, n + 1, nnz_item, batch * nnz_item, idx, algo=algo,
-                     keep=(crow, col))
-    pat._uniform = _uniform_from(max_row, batch * n, batch * nnz_item)
-    pat.extras["window"] = plan
+    pat, _ = _new_pattern(crow_c, col_c, None, batch, n, m, n + 1, nnz_item, batch * nnz_item, idx, keep=(crow, col))
     pat.cache_key = key
     _cache_put(key, pat, (crow, col))
     return pat
@@ -591,6 +581,14 @@ class CooPattern:
     nnz_unique: int
     fingerprint: Optional[torch.Tensor] = field(default=None, repr=False)
     cache_key: Optional[tuple] = field(default=None, repr=False)
+
+    @property
+    def nnz_out(self) -> int:
+        return self.nnz_unique
+
+    def values(self, A: torch.Tensor) -> torch.Tensor:
+        vals = aligned_contiguous(A._values())
+        return vals if self.seg is None else _ops.segment_sum_values(vals, self.sort_perm, self.seg, self.nnz_unique)
 
 
 def _sort_coo(indices: torch.Tensor, dims, key_dims: int, perm_idx: int, want_sorted: bool):
@@ -622,44 +620,42 @@ def _coo_to_flat_csr(indices: torch.Tensor, batch: int, n: int, m: int, perm: Op
         nat.check(nat.lib().tsgu_coo_to_csr(nat.ptr(indices), ndim, nnz, indices.stride(0), batch, n, nat.ptr(perm),
                                             nat.ptr(rowptr), nat.ptr(colind), idx, nat.stream_ptr(dev)),
                   "tsgu_coo_to_csr")
-    algo, plan, _, max_row = _analyse(rowptr, colind, batch, n, m, n, 0, nnz, idx)
-    pat = CsrPattern(rowptr, colind, perm, batch, n, m, n, 0, nnz, idx, algo=algo, keep=keep)
-    pat._uniform = _uniform_from(max_row, batch * n, nnz)
-    pat.extras["window"] = plan
-    return pat
+    return _new_pattern(rowptr, colind, perm, batch, n, m, n, 0, nnz, idx, keep=keep)[0]
 
 
-def coo_pattern(A: torch.Tensor) -> CooPattern:
-    """COO -> kernel-ready structure (sort + rowptr), cached per index tensor."""
+def coo_pattern(A: torch.Tensor, unique: bool = False) -> CooPattern:
+    """COO -> kernel-ready structure (sort + rowptr), cached per index tensor.
+
+    Duplicates of a batched tensor are coalesced onto its sorted unique pattern, as the reference does.  Those of an
+    uncoalesced 2-D tensor stay separate entries, which a product may keep, unless `unique`: a triangular solve may not,
+    its diagonal must be one value."""
     ind = A._indices()
     coalesced = A.is_coalesced()
-    key = ("coo", _index_key(ind), tuple(A.shape), coalesced, ind.device)
+    batched = A.dim() == 3
+    unique = unique and not (batched or coalesced)
+    if unique:
+        key = ("coo-unique", _index_key(ind), tuple(A.shape), ind.device)
+    else:
+        key = ("coo", _index_key(ind), tuple(A.shape), coalesced, ind.device)
     hit = _cache_get(key, (ind,))
     if hit is not None:
         return hit
     ind_key = ind
     if ind.stride(1) != 1:
         ind = ind.contiguous()
-    batched = A.dim() == 3
     batch = A.shape[0] if batched else 1
     n, m = A.shape[-2], A.shape[-1]
     nnz = ind.shape[1]
     idx = _internal_idx(batch, n, m, nnz)
-    if not batched:
-        if coalesced:  # already sorted and unique: no sort, identity value map
-            csr = _coo_to_flat_csr(ind, 1, n, m, None, idx, keep=(ind,))
-            pat = CooPattern(csr, None, None, None, None, nnz)
-        else:  # stable sort by row only: entries of a row keep storage order, duplicates just add up
-            perm, _ = _sort_coo(ind, (n, m), 1, idx, False)
-            csr = _coo_to_flat_csr(ind, 1, n, m, perm, idx, keep=(ind,))
-            pat = CooPattern(csr, perm, None, None, None, nnz)
-    else:
-        dims = (batch, n, m)
-        if coalesced:
-            csr = _coo_to_flat_csr(ind, batch, n, m, None, idx, keep=(ind,))
-            pat = CooPattern(csr, None, ind, None, None, nnz)
-        else:
-            pat = _coo_unique(ind, dims, batch, n, m, idx)
+    if coalesced:  # already sorted and unique: no sort, identity value map
+        csr = _coo_to_flat_csr(ind, batch, n, m, None, idx, keep=(ind,))
+        pat = CooPattern(csr, None, ind if batched else None, None, None, nnz)
+    elif batched or unique:
+        pat = _coo_unique(ind, (batch, n, m) if batched else (n, m), batch, n, m, idx)
+    else:  # stable sort by row only: entries of a row keep storage order, duplicates just add up
+        perm, _ = _sort_coo(ind, (n, m), 1, idx, False)
+        csr = _coo_to_flat_csr(ind, 1, n, m, perm, idx, keep=(ind,))
+        pat = CooPattern(csr, perm, None, None, None, nnz)
     pat.cache_key = key
     _cache_put(key, pat, (ind_key,))
     return pat
@@ -687,25 +683,37 @@ def _coo_unique(ind: torch.Tensor, dims, batch: int, n: int, m: int, idx: int) -
     return CooPattern(csr, None, uniq, seg, perm, uniq.shape[1])
 
 
-def coo_unique_pattern(A: torch.Tensor) -> CooPattern:
-    """Pattern of a COO tensor with duplicates coalesced, also for 2-D input (``coo_pattern`` keeps the duplicates of
-    an uncoalesced 2-D tensor as separate entries, which a product may, but a triangular solve may not: its diagonal
-    must be one value).  Same cache as ``coo_pattern``."""
-    if A.dim() == 3 or A.is_coalesced():
-        return coo_pattern(A)
-    ind = A._indices()
-    key = ("coo-unique", _index_key(ind), tuple(A.shape), ind.device)
-    hit = _cache_get(key, (ind,))
-    if hit is not None:
-        return hit
-    ind_key = ind
-    if ind.stride(1) != 1:
-        ind = ind.contiguous()
-    n, m = A.shape
-    pat = _coo_unique(ind, (n, m), 1, n, m, _internal_idx(1, n, m, ind.shape[1]))
-    pat.cache_key = key
-    _cache_put(key, pat, (ind_key,))
-    return pat
+# ------------------------------------------------------------------------------------------ operands
+def pattern_of(A: torch.Tensor, unique: bool = False):
+    """A's cached pattern (built on first use): a CsrPattern for CSR input, a CooPattern for COO (``unique``: see
+    :func:`coo_pattern`).  Both answer what an operator needs without looking at A's layout again:
+
+    * ``.csr`` -- the flat CsrPattern the kernels read;
+    * ``.values(A)`` -- A's values in the order those kernels index them: aligned and contiguous, in storage order
+      (a kernel reads them through ``csr.perm`` where the pattern has one), summed onto the unique pattern where
+      duplicates were coalesced;
+    * ``.out_index`` / ``.nnz_out`` -- where the SDDMM over ``.csr`` writes entry e and how many values it writes,
+      and ``.grad_indices`` -- the COO indices those values sit on (None: A's own), for :func:`sparse_like`."""
+    if A.layout == torch.sparse_csr:
+        return csr_pattern(A)
+    if A.layout == torch.sparse_coo:
+        return coo_pattern(A, unique)
+    raise ValueError("A should be in either COO or CSR sparse format")
+
+
+def sparse_values(A: torch.Tensor) -> torch.Tensor:
+    """The stored values of a CSR or COO tensor, in storage order."""
+    return A.values() if A.layout == torch.sparse_csr else A._values()
+
+
+def sparse_like(A: torch.Tensor, values: torch.Tensor, indices: Optional[torch.Tensor] = None,
+                is_coalesced: Optional[bool] = None) -> torch.Tensor:
+    """A sparse tensor with A's layout and shape holding `values`: on A's own crow/col (CSR), or on A's indices or the
+    given ones (COO, with the given coalesced flag)."""
+    if A.layout == torch.sparse_csr:
+        return torch.sparse_csr_tensor(A.crow_indices(), A.col_indices(), values.view(A.values().shape), A.shape)
+    return torch.sparse_coo_tensor(A._indices() if indices is None else indices, values, A.shape,
+                                   is_coalesced=is_coalesced)
 
 
 def prepare_pattern(A: torch.Tensor, backward: bool = True, reuse: bool = True) -> None:
@@ -718,12 +726,6 @@ def prepare_pattern(A: torch.Tensor, backward: bool = True, reuse: bool = True) 
 
     `reuse` says the pattern will serve many steps, so the transposed structure gets its layout optimisations right
     away (``CsrPattern.transpose``); pass False for a pattern that lives for a single step."""
-    if A.layout == torch.sparse_csr:
-        csr = csr_pattern(A)
-    elif A.layout == torch.sparse_coo:
-        csr = coo_pattern(A).csr
-    else:
-        raise ValueError("A should be in either COO or CSR sparse format")
-    window_plan(csr)
+    csr = pattern_of(A).csr
     if backward:
         csr.transpose(optimise=True if reuse else False)

@@ -32,6 +32,7 @@ import torch.distributed as dist
 import os
 
 from . import _native
+from ._pattern import sparse_like, sparse_values
 from .sparse_matmul import SparseMatMul, _grad_A, _grad_B, sparse_mm
 
 _OVERLAP_SM_MARGIN = int(os.environ.get("TSGU_B200_OVERLAP_SM_MARGIN", "20"))
@@ -225,10 +226,6 @@ def k_shard_bounds(K: int, world: int, rank: int, align: int = 1) -> Tuple[int, 
     return min(lo, K), min(hi, K)
 
 
-def _sparse_values(t: torch.Tensor) -> torch.Tensor:
-    return t.values() if t.layout == torch.sparse_csr else t._values()
-
-
 class _AllReduceSparseGrad(torch.autograd.Function):
     """Identity on a sparse operand in forward; sums the gradient's stored values over the group in backward
     (gloo / injected-operator path of :func:`sparse_mm_k_sharded`)."""
@@ -247,11 +244,9 @@ class _AllReduceSparseGrad(torch.autograd.Function):
             return g, None
         if grad.layout == torch.sparse_coo and not grad.is_coalesced():
             grad = grad.coalesce()
-        v = _sparse_values(grad).contiguous()
+        v = sparse_values(grad).contiguous()
         dist.all_reduce(v, op=dist.ReduceOp.SUM, group=ctx.group)
-        if grad.layout == torch.sparse_csr:
-            return torch.sparse_csr_tensor(grad.crow_indices(), grad.col_indices(), v, grad.shape), None
-        return torch.sparse_coo_tensor(grad._indices(), v, grad.shape, is_coalesced=True), None
+        return sparse_like(grad, v, is_coalesced=True), None
 
 
 class _KShardedMatMul(torch.autograd.Function):
@@ -269,7 +264,7 @@ class _KShardedMatMul(torch.autograd.Function):
         gradA = work = None
         if ctx.needs_input_grad[0]:
             gradA = _grad_A(ctx, grad)
-            work = dist.all_reduce(_sparse_values(gradA), op=dist.ReduceOp.SUM, group=ctx.group, async_op=True)
+            work = dist.all_reduce(sparse_values(gradA), op=dist.ReduceOp.SUM, group=ctx.group, async_op=True)
         gradB = _grad_B(ctx, grad) if ctx.needs_input_grad[1] else None
         if work is not None:
             work.wait()

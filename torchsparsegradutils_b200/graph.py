@@ -11,7 +11,7 @@ from typing import Tuple
 
 import torch
 
-from ._pattern import coo_pattern, csr_pattern, pin_pattern
+from ._pattern import pattern_of, pin_pattern, sparse_like, sparse_values
 from .sparse_matmul import sparse_mm
 
 
@@ -28,13 +28,9 @@ class GraphedSparseMM:
         if not (A.is_cuda and B.is_cuda and G.is_cuda):
             raise RuntimeError("GraphedSparseMM needs CUDA tensors")
         dev = B.device
-        self._csr = A.layout == torch.sparse_csr
         with torch.no_grad():
-            if self._csr:
-                A_static = torch.sparse_csr_tensor(A.crow_indices(), A.col_indices(), A.values().clone(), A.shape)
-            else:
-                A_static = torch.sparse_coo_tensor(A._indices(), A._values().clone(), A.shape,
-                                                   is_coalesced=A.is_coalesced())
+            A_static = sparse_like(A, sparse_values(A).clone(),
+                                   is_coalesced=A.is_coalesced() if A.layout == torch.sparse_coo else None)
         self._A = A_static.requires_grad_(True)
         self._B = B.detach().clone().contiguous().requires_grad_(True)
         self._G = G.detach().clone().contiguous()
@@ -52,25 +48,22 @@ class GraphedSparseMM:
             # The pattern builds (sort / transpose, with their host syncs) are not capturable: build the pattern
             # here and PIN it to this object, so the capture below -- and nothing later -- depends on what the
             # LRU pattern cache happens to hold (it may have capacity 0, or evict the entry between steps).
-            self._pattern = csr_pattern(self._A) if self._csr else coo_pattern(self._A)
+            self._pattern = pattern_of(self._A)
             pin_pattern(self._pattern.cache_key, self._pattern)
-            (self._pattern if self._csr else self._pattern.csr).transpose(optimise=True)  # final layout before capture
+            self._pattern.csr.transpose(optimise=True)  # final layout before capture
             for _ in range(max(warmup, 1)):
                 step()
         torch.cuda.current_stream(dev).wait_stream(side)
         self._graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self._graph):
             self._C = step()
-        gA = self._A.grad
-        self._gA_values = gA.values() if self._csr else gA._values()
+        self._gA_values = sparse_values(self._A.grad)
         self._gB = self._B.grad
-
-    def _values(self) -> torch.Tensor:
-        return self._A.values() if self._csr else self._A._values()
 
     @torch.no_grad()
     def __call__(self, values: torch.Tensor, B: torch.Tensor, G: torch.Tensor) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
-        self._values().copy_(values.reshape(self._values().shape))
+        A_values = sparse_values(self._A)
+        A_values.copy_(values.reshape(A_values.shape))
         self._B.copy_(B)
         self._G.copy_(G)
         self._graph.replay()

@@ -11,7 +11,7 @@ from __future__ import annotations
 import torch
 
 from . import _ops
-from ._pattern import csr_pattern
+from ._pattern import csr_pattern, pattern_of, sparse_like
 
 
 def sddmm(A: torch.Tensor, X: torch.Tensor, Y: torch.Tensor) -> torch.Tensor:
@@ -25,14 +25,7 @@ def sddmm(A: torch.Tensor, X: torch.Tensor, Y: torch.Tensor) -> torch.Tensor:
     """
     if A.layout not in (torch.sparse_coo, torch.sparse_csr):
         raise ValueError("A should be in either COO or CSR sparse format")
-    if not (A.is_cuda and X.is_cuda and Y.is_cuda):
-        raise RuntimeError("torchsparsegradutils_b200.sddmm runs on CUDA tensors only; there is no CPU fallback")
-    if X.dim() != A.dim() or Y.dim() != A.dim():
-        raise ValueError("A, X and Y must all be 2D or all be 3D tensors")
-    if X.size(-2) != A.size(-2) or Y.size(-2) != A.size(-1) or X.size(-1) != Y.size(-1):
-        raise ValueError(f"Incompatible shapes: A {tuple(A.shape)}, X {tuple(X.shape)}, Y {tuple(Y.shape)}")
-    if X.dtype != Y.dtype:
-        raise RuntimeError(f"sddmm: X and Y must have the same dtype, got {X.dtype} and {Y.dtype}")
+    _check_operands(A, X, Y)
     X, Y = X.detach(), Y.detach()
     if A.layout == torch.sparse_coo:
         if A.dim() != 2 or A.sparse_dim() != 2:
@@ -42,6 +35,17 @@ def sddmm(A: torch.Tensor, X: torch.Tensor, Y: torch.Tensor) -> torch.Tensor:
     pat = csr_pattern(A)
     out = _ops.sddmm(pat, X, Y, None, pat.nnz_total)
     return out.view(A.values().shape)
+
+
+def _check_operands(A: torch.Tensor, X: torch.Tensor, Y: torch.Tensor) -> None:
+    if not (A.is_cuda and X.is_cuda and Y.is_cuda):
+        raise RuntimeError("torchsparsegradutils_b200.sddmm runs on CUDA tensors only; there is no CPU fallback")
+    if X.dim() != A.dim() or Y.dim() != A.dim():
+        raise ValueError("A, X and Y must all be 2D or all be 3D tensors")
+    if X.size(-2) != A.size(-2) or Y.size(-2) != A.size(-1) or X.size(-1) != Y.size(-1):
+        raise ValueError(f"Incompatible shapes: A {tuple(A.shape)}, X {tuple(X.shape)}, Y {tuple(Y.shape)}")
+    if X.dtype != Y.dtype:
+        raise RuntimeError(f"sddmm: X and Y must have the same dtype, got {X.dtype} and {Y.dtype}")
 
 
 def solve_grad_A(A: torch.Tensor, gradB: torch.Tensor, x: torch.Tensor, transpose: bool = False) -> torch.Tensor:
@@ -73,9 +77,7 @@ def solve_grad_A(A: torch.Tensor, gradB: torch.Tensor, x: torch.Tensor, transpos
     vals = vals.neg_()
     if vals.dtype != A.dtype:
         vals = vals.to(A.dtype)
-    if A.layout == torch.sparse_coo:
-        return torch.sparse_coo_tensor(A._indices(), vals, A.shape)
-    return torch.sparse_csr_tensor(A.crow_indices(), A.col_indices(), vals, A.shape)
+    return sparse_like(A, vals)
 
 
 # ----------------------------------------------------------------- batched plumbing of the solves (SURVEY 8(f) rank 4)
@@ -97,17 +99,10 @@ def block_diag_operand(A: torch.Tensor) -> torch.Tensor:
     if A.layout == torch.sparse_csr:
         crow, col = _ops.block_diag_csr(A.crow_indices(), A.col_indices(), m)
         return torch.sparse_csr_tensor(crow, col, A.values().reshape(-1), (b * n, b * m))
-    if A.layout != torch.sparse_coo:
-        raise ValueError("A should be in either COO or CSR sparse format")
-    from ._pattern import coo_pattern
-
-    pat = coo_pattern(A)  # flat CSR over b*n rows, item-local columns, duplicates coalesced like the reference (:580)
-    csr = pat.csr
-    vals = A._values()
-    if pat.seg is not None:
-        vals = _ops.segment_sum_values(vals.contiguous(), pat.sort_perm, pat.seg, pat.nnz_unique)
-    elif csr.perm is not None:
-        vals = _ops.gather_values(vals.contiguous(), csr.perm)
+    pat = pattern_of(A)  # COO: flat CSR over b*n rows, item-local columns, duplicates coalesced like the reference (:580)
+    csr, vals = pat.csr, pat.values(A)
+    if csr.perm is not None:
+        vals = _ops.gather_values(vals, csr.perm)
     rows = torch.arange(b * n, device=A.device, dtype=csr.rowptr.dtype)
     item_of_entry = torch.repeat_interleave(rows // n, (csr.rowptr[1:] - csr.rowptr[:-1]).long())
     col = csr.colind.long() + item_of_entry.long() * m
@@ -123,15 +118,11 @@ def _solve_grad_A_batched(A: torch.Tensor, gradB: torch.Tensor, x: torch.Tensor,
     b, n, m = A.shape
     gradB = gradB.reshape(b, n, -1) if gradB.dim() != 3 else gradB
     x = x.reshape(b, m, -1) if x.dim() != 3 else x
-    if A.layout == torch.sparse_csr:
-        vals = sddmm(A, x, gradB) if transpose else sddmm(A, gradB, x)
-        return torch.sparse_csr_tensor(A.crow_indices(), A.col_indices(), vals.neg_(), A.shape)
-    from ._pattern import coo_pattern
-
-    pat = coo_pattern(A)
     G, Y = (x, gradB) if transpose else (gradB, x)
-    vals = _ops.sddmm(pat.csr, G.detach(), Y.detach(), None, pat.nnz_unique).neg_()
-    return torch.sparse_coo_tensor(pat.grad_indices, vals, A.shape, is_coalesced=True)
+    _check_operands(A, G, Y)
+    pat = pattern_of(A)
+    vals = _ops.sddmm(pat.csr, G.detach(), Y.detach(), pat.out_index, pat.nnz_out).neg_()
+    return sparse_like(A, vals, pat.grad_indices, is_coalesced=True)
 
 
 def lstsq_grad_A(A: torch.Tensor, gradB: torch.Tensor, x: torch.Tensor, B: torch.Tensor, Apgb: torch.Tensor) -> torch.Tensor:
@@ -152,6 +143,4 @@ def lstsq_grad_A(A: torch.Tensor, gradB: torch.Tensor, x: torch.Tensor, B: torch
     with torch.no_grad():
         resid = B - sparse_mm(A.detach(), x.detach())
     vals = sddmm(A, resid, Apgb).sub_(sddmm(A, gradB, x))
-    if A.layout == torch.sparse_coo:
-        return torch.sparse_coo_tensor(A._indices(), vals, A.shape)
-    return torch.sparse_csr_tensor(A.crow_indices(), A.col_indices(), vals, A.shape)
+    return sparse_like(A, vals)

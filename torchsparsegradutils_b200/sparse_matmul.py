@@ -25,7 +25,7 @@ from typing import cast
 import torch
 
 from . import _native, _ops
-from ._pattern import CooPattern, CsrPattern, aligned_contiguous, coo_pattern, csr_pattern
+from ._pattern import pattern_of, sparse_like
 
 
 def sparse_mm(A: torch.Tensor, B: torch.Tensor) -> torch.Tensor:
@@ -53,6 +53,12 @@ def sparse_mm(A: torch.Tensor, B: torch.Tensor) -> torch.Tensor:
         Non-CUDA tensors, mismatching dtypes/devices, unsupported dtype, or a kernel failure.
         There is no CPU fallback.
     """
+    _check_args(A, B)
+    return cast(torch.Tensor, SparseMatMul.apply(A, B))
+
+
+def _check_args(A: torch.Tensor, B: torch.Tensor, square: bool = False) -> None:
+    """The ValueError checks of sparse_mm (`square`: and of sparse_triangular_solve), in the reference's order."""
     if not isinstance(A, torch.Tensor) or not isinstance(B, torch.Tensor):
         raise ValueError("Both A and B should be instances of torch.Tensor")
     if A.dim() < 2 or B.dim() < 2:
@@ -65,24 +71,27 @@ def sparse_mm(A: torch.Tensor, B: torch.Tensor) -> torch.Tensor:
         raise ValueError("B must be a dense (strided) tensor")
     if A.dim() == 3 and A.size(0) != B.size(0):
         raise ValueError("If batched, A and B must have the same batch size")
+    if square and A.size(-1) != A.size(-2):
+        raise ValueError(f"A must be square, got A[..., {A.size(-2)}, {A.size(-1)}]")
     if A.size(-1) != B.size(-2):
         raise ValueError(f"Incompatible inner dimensions: A[..., {A.size(-1)}] vs B[..., {B.size(-2)}]")
 
-    return cast(torch.Tensor, SparseMatMul.apply(A, B))
 
-
-def _check_runtime(A: torch.Tensor, B: torch.Tensor) -> None:
+def _check_runtime(A: torch.Tensor, B: torch.Tensor, op: str = "sparse_mm", float_only: bool = False) -> None:
+    """The RuntimeError checks of `op`; `float_only`: values must be float32 / float64 (no bfloat16)."""
     if not (A.is_cuda and B.is_cuda):
         raise RuntimeError(
-            "torchsparsegradutils_b200.sparse_mm runs on CUDA (sm_100a) tensors only; got "
+            f"torchsparsegradutils_b200.{op} runs on CUDA (sm_100a) tensors only; got "
             f"A on {A.device}, B on {B.device}. There is no CPU fallback.")
     if A.device != B.device:
-        raise RuntimeError(f"sparse_mm: A and B must be on the same device, got {A.device} and {B.device}")
+        raise RuntimeError(f"{op}: A and B must be on the same device, got {A.device} and {B.device}")
     if A.dtype != B.dtype:
-        raise RuntimeError(f"sparse_mm: A and B must have the same dtype, got {A.dtype} and {B.dtype}")
+        raise RuntimeError(f"{op}: A and B must have the same dtype, got {A.dtype} and {B.dtype}")
+    if float_only and B.dtype not in (torch.float32, torch.float64):
+        raise RuntimeError(f"{op}: unsupported value dtype {B.dtype}; supported: float32, float64")
     _native.val_enum(B.dtype)  # RuntimeError("unsupported value dtype ...") for float16 / complex / integer operands
     if A.layout == torch.sparse_coo and (A.sparse_dim() != A.dim() or A.dense_dim() != 0):
-        raise RuntimeError("sparse_mm: COO input must have sparse_dim == ndim and no dense dimensions")
+        raise RuntimeError(f"{op}: COO input must have sparse_dim == ndim and no dense dimensions")
 
 
 class SparseMatMul(torch.autograd.Function):
@@ -97,26 +106,17 @@ class SparseMatMul(torch.autograd.Function):
         # remember a non-contiguous (but dense) layout of B so grad_B can be handed back in it
         ctx.B_strides = B.stride() if (not B.is_contiguous() and _ops.is_dense_non_overlapping(B)) else None
         A, B = A.detach(), B.detach()
-
-        coalesced_vals = None
-        if A.layout == torch.sparse_csr:
-            pat = csr_pattern(A)
-            csr, vals = pat, aligned_contiguous(A.values())
-        else:
-            pat = coo_pattern(A)
-            csr, vals = pat.csr, aligned_contiguous(A._values())
-            if pat.seg is not None:  # batched COO with duplicates: coalesce values onto the unique pattern
-                coalesced_vals = _ops.segment_sum_values(vals, pat.sort_perm, pat.seg, pat.nnz_unique)
-                vals = coalesced_vals
+        pat = pattern_of(A)
+        vals = pat.values(A)
 
         # a strided view of B (eps.t(), permute(1,2,0) from _batch_sparse_mv) is packed once here and the
         # packed copy is what backward's SDDMM re-reads -- the reference re-copies it as well (:153)
         Bk = _ops.prepare_dense(B if ctx.batched else B.unsqueeze(0))
-        x = _ops.spmm(csr, vals, Bk, tag="spmm_fwd")
+        x = _ops.spmm(pat.csr, vals, Bk, tag="spmm_fwd")
         x = x if ctx.batched else x[0]
 
         ctx.pattern = pat
-        ctx.save_for_backward(A, Bk, *(() if coalesced_vals is None else (coalesced_vals,)))
+        ctx.save_for_backward(A, Bk, vals)
         return x
 
     @staticmethod
@@ -138,9 +138,7 @@ _side_streams: dict = {}
 
 
 def _concurrent_backward_pays(ctx, grad) -> bool:
-    pat = ctx.pattern
-    csr = pat if isinstance(pat, CsrPattern) else pat.csr
-    return 0 < csr.nnz_total * grad.shape[-1] * grad.element_size() <= _CONCURRENT_BWD_MAX_GATHER_BYTES
+    return 0 < ctx.pattern.csr.nnz_total * grad.shape[-1] * grad.element_size() <= _CONCURRENT_BWD_MAX_GATHER_BYTES
 
 
 def _backward_two_streams(ctx, grad):
@@ -149,10 +147,9 @@ def _backward_two_streams(ctx, grad):
     side = _side_streams.get(dev.index)
     if side is None:
         side = _side_streams[dev.index] = torch.cuda.Stream(dev)
-    pat = ctx.pattern
     # a transposed structure that must still be built (or get its layout upgrade) is built HERE: tensors a cached
     # pattern owns are allocated -- and the ones it replaces freed -- under the caller's stream, never the side stream
-    patT = (pat if isinstance(pat, CsrPattern) else pat.csr).transpose()
+    patT = ctx.pattern.csr.transpose()
     side.wait_stream(main)  # fork (under graph capture: a parallel branch of the graph)
     with torch.cuda.stream(side):
         gradB = _grad_B(ctx, grad, patT)
@@ -164,39 +161,22 @@ def _backward_two_streams(ctx, grad):
 
 def _grad_A(ctx, grad):
     """grad_A[e] = <grad[i_e, :], B[j_e, :]> on A's pattern only (reference sparse_matmul.py:173-219)."""
-    saved = ctx.saved_tensors
-    A, B = saved[0], saved[1]
+    A, B = ctx.saved_tensors[:2]
     pat = ctx.pattern
-    if isinstance(pat, CsrPattern):
-        v = _ops.sddmm(pat, grad, B, None, pat.nnz_total)
-        return torch.sparse_csr_tensor(A.crow_indices(), A.col_indices(), v.view(A.values().shape), A.shape)
-    csr = cast(CooPattern, pat).csr
-    if not ctx.batched:
-        # per stored entry, in storage order (duplicates each get the full dot product)
-        v = _ops.sddmm(csr, grad, B, pat.out_index, csr.nnz_total)
-        return torch.sparse_coo_tensor(A._indices(), v, A.shape)
-    # batched COO: the gradient lives on the sorted unique pattern (reference :213-217)
-    v = _ops.sddmm(csr, grad, B, None, pat.nnz_unique)
-    return torch.sparse_coo_tensor(pat.grad_indices, v, A.shape)
+    # 2-D COO: per stored entry, in storage order (duplicates each get the full dot product); batched COO: on the
+    # sorted unique pattern (reference :213-217)
+    v = _ops.sddmm(pat.csr, grad, B, pat.out_index, pat.nnz_out)
+    return sparse_like(A, v, pat.grad_indices)
 
 
 def _grad_B(ctx, grad, patT=None):
     """grad_B = A^T grad through the cached transposed structure (reference sparse_matmul.py:222-232)."""
-    saved = ctx.saved_tensors
-    A = saved[0]
-    pat = ctx.pattern
-    is_csr = isinstance(pat, CsrPattern)
-    csr = pat if is_csr else cast(CooPattern, pat).csr
-    if len(saved) > 2:
-        vals = saved[2]
-    elif is_csr:
-        vals = aligned_contiguous(A.values())
-    else:
-        vals = aligned_contiguous(A._values())
+    vals = ctx.saved_tensors[2]
     want = None
     if ctx.B_strides is not None:  # ask for B's own layout; kernels that can write it directly save the re-stride pass
         want = tuple(ctx.B_strides) if ctx.batched else (ctx.B_shape[0] * ctx.B_shape[1],) + tuple(ctx.B_strides)
-    gradB = _ops.spmm(csr.transpose() if patT is None else patT, vals, grad, tag="spmm_gradB", out_strides=want)
+    patT = ctx.pattern.csr.transpose() if patT is None else patT
+    gradB = _ops.spmm(patT, vals, grad, tag="spmm_gradB", out_strides=want)
     gradB = gradB if ctx.batched else gradB[0]
     if ctx.B_strides is not None and tuple(gradB.stride()) != tuple(ctx.B_strides):
         gradB = _ops.restride_like(gradB, ctx.B_shape, ctx.B_strides)

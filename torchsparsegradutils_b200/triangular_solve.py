@@ -26,9 +26,9 @@ import torch
 
 from . import _native as nat
 from . import _ops
-from ._pattern import (CsrPattern, TriPlan, _internal_idx, _sort_coo, aligned_contiguous, coo_unique_pattern,
-                       csr_pattern)
+from ._pattern import CsrPattern, TriPlan, _sort_coo, _transpose_csr, pattern_of
 from .sddmm import solve_grad_A
+from .sparse_matmul import _check_args, _check_runtime
 
 
 def sparse_triangular_solve(A: torch.Tensor, B: torch.Tensor, upper: bool = True, unitriangular: bool = False,
@@ -62,50 +62,8 @@ def sparse_triangular_solve(A: torch.Tensor, B: torch.Tensor, upper: bool = True
         Non-CUDA tensors, mismatching dtypes/devices, a dtype other than float32 / float64, or a kernel failure.
         There is no CPU fallback.
     """
-    if not isinstance(A, torch.Tensor) or not isinstance(B, torch.Tensor):
-        raise ValueError("Both A and B should be instances of torch.Tensor")
-    if A.dim() < 2 or B.dim() < 2:
-        raise ValueError("Both A and B should be at least 2-dimensional tensors")
-    if A.dim() != B.dim() or A.dim() not in (2, 3):
-        raise ValueError("A and B must both be 2D or both be 3D tensors")
-    if A.layout not in {torch.sparse_coo, torch.sparse_csr}:
-        raise ValueError("A should be in either COO or CSR sparse format")
-    if B.layout != torch.strided:
-        raise ValueError("B must be a dense (strided) tensor")
-    if A.dim() == 3 and A.size(0) != B.size(0):
-        raise ValueError("If batched, A and B must have the same batch size")
-    if A.size(-1) != A.size(-2):
-        raise ValueError(f"A must be square, got A[..., {A.size(-2)}, {A.size(-1)}]")
-    if A.size(-1) != B.size(-2):
-        raise ValueError(f"Incompatible inner dimensions: A[..., {A.size(-1)}] vs B[..., {B.size(-2)}]")
-
+    _check_args(A, B, square=True)
     return cast(torch.Tensor, SparseTriangularSolve.apply(A, B, bool(upper), bool(unitriangular), bool(transpose)))
-
-
-def _check_runtime(A: torch.Tensor, B: torch.Tensor) -> None:
-    if not (A.is_cuda and B.is_cuda):
-        raise RuntimeError(
-            "torchsparsegradutils_b200.sparse_triangular_solve runs on CUDA (sm_100a) tensors only; got "
-            f"A on {A.device}, B on {B.device}. There is no CPU fallback.")
-    if A.device != B.device:
-        raise RuntimeError(f"sparse_triangular_solve: A and B must be on the same device, got {A.device} and {B.device}")
-    if A.dtype != B.dtype:
-        raise RuntimeError(f"sparse_triangular_solve: A and B must have the same dtype, got {A.dtype} and {B.dtype}")
-    if B.dtype not in (torch.float32, torch.float64):
-        raise RuntimeError(f"sparse_triangular_solve: unsupported value dtype {B.dtype}; supported: float32, float64")
-    if A.layout == torch.sparse_coo and (A.sparse_dim() != A.dim() or A.dense_dim() != 0):
-        raise RuntimeError("sparse_triangular_solve: COO input must have sparse_dim == ndim and no dense dimensions")
-
-
-def _operand(A: torch.Tensor):
-    """(flat CSR pattern, value array its plans index) of A; COO duplicates are summed here."""
-    if A.layout == torch.sparse_csr:
-        return csr_pattern(A), aligned_contiguous(A.values()).reshape(-1)
-    pat = coo_unique_pattern(A)
-    vals = aligned_contiguous(A._values())
-    if pat.seg is not None:
-        vals = _ops.segment_sum_values(vals, pat.sort_perm, pat.seg, pat.nnz_unique)
-    return pat.csr, vals  # a sort permutation (pat.csr.perm) is folded into the plan's value positions
 
 
 class SparseTriangularSolve(torch.autograd.Function):
@@ -113,11 +71,12 @@ class SparseTriangularSolve(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, A, B, upper, unitriangular, transpose):
-        _check_runtime(A, B)
+        _check_runtime(A, B, "sparse_triangular_solve", float_only=True)
         ctx.batched = B.dim() == 3
         ctx.flags = (upper, unitriangular, transpose)
         A, B = A.detach(), B.detach()
-        csr, vals = _operand(A)
+        pat = pattern_of(A, unique=True)  # COO duplicates are summed
+        csr, vals = pat.csr, pat.values(A)  # a sort permutation (csr.perm) is folded into the plan's value positions
         x = _solve(csr, vals, B if ctx.batched else B.unsqueeze(0), upper, unitriangular, transpose)
         x = x if ctx.batched else x[0]
         ctx.pattern = csr
@@ -143,13 +102,7 @@ def solve_plan(A: torch.Tensor, upper: bool = True, transpose: bool = False) -> 
 
     Call it ahead of the first solve to take the one-off analysis (one host read) out of the first step, e.g. before a
     ``torch.cuda.graph`` capture; ``.levels`` is the number of dependent steps of the solve."""
-    if A.layout == torch.sparse_csr:
-        csr = csr_pattern(A)
-    elif A.layout == torch.sparse_coo:
-        csr = coo_unique_pattern(A).csr
-    else:
-        raise ValueError("A should be in either COO or CSR sparse format")
-    return _plan(csr, upper, transpose)
+    return _plan(pattern_of(A, unique=True).csr, upper, transpose)
 
 
 def _plan(csr: CsrPattern, upper: bool, transpose: bool) -> TriPlan:
@@ -162,33 +115,12 @@ def _plan(csr: CsrPattern, upper: bool, transpose: bool) -> TriPlan:
     return plan
 
 
-def _transposed(csr: CsrPattern):
-    """CSR of the transposes straight from tsgu_csr_transpose (flat, stable, no length sorting or padding: the solve
-    plan orders rows by level itself).  Returns (rowptr, colind, perm into the value array, idx)."""
-    dev = csr.device
-    idx = _internal_idx(csr.batch, csr.m, csr.n, csr.nnz_total)
-    odt = nat.IDX_TORCH[idx]
-    rowptr = torch.empty(csr.batch * csr.m + 1, dtype=odt, device=dev)
-    colind = torch.empty(csr.nnz_total, dtype=odt, device=dev)
-    perm = torch.empty(csr.nnz_total, dtype=odt, device=dev)
-    L = nat.lib()
-    with torch.cuda.device(dev):
-        ws = nat.workspace(L.tsgu_csr_transpose_workspace_bytes(csr.batch, csr.m, csr.nnz_total, idx), dev)
-        nat.check(L.tsgu_csr_transpose(nat.ptr(csr.rowptr), nat.ptr(csr.colind), csr.batch, csr.n, csr.m,
-                                       csr.rowptr_bstride, csr.nnz_bstride, csr.nnz_total, csr.idx, nat.ptr(rowptr),
-                                       nat.ptr(colind), nat.ptr(perm), idx, nat.ptr(ws), ws.numel(),
-                                       nat.stream_ptr(dev)), "tsgu_csr_transpose")
-    if csr.perm is not None and csr.nnz_total > 0:
-        perm = csr.perm.to(odt).index_select(0, perm.long())
-    return rowptr, colind, perm, idx
-
-
 def _build_plan(csr: CsrPattern, lower: bool, transpose: bool) -> TriPlan:
     dev = csr.device
     batch, n = csr.batch, csr.n
     rows = batch * n
     if transpose:
-        rowptr, colind, perm, idx = _transposed(csr)
+        rowptr, colind, perm, idx = _transpose_csr(csr)
         rbs, nbs = n, 0
     else:
         rowptr, colind, perm, idx = csr.rowptr, csr.colind, csr.perm, csr.idx
