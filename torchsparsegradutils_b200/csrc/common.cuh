@@ -5,9 +5,14 @@
 #include <stdint.h>
 #include <stdlib.h>
 
+#include <type_traits>
+
 #include "../../include/tsgu_b200.h"
 
 namespace tsgu {
+
+template <int N>
+using Int = std::integral_constant<int, N>;
 
 // ---------------------------------------------------------------- launch accounting
 extern unsigned long long g_launches;  // defined in api.cu
@@ -27,6 +32,31 @@ extern thread_local int g_sm_margin;  // defined in api.cu
 inline int64_t persistent_sms() {
   const int m = g_sm_margin;
   return m > 0 && m < kNumSMs ? kNumSMs - m : kNumSMs;
+}
+
+// Persistent kernels (CTA b walks tiles b, b + gridDim.x, ...).  persistent_ctas() lets `kern` use `smem` bytes of
+// dynamic shared memory and leaves its resident CTAs per SM in `ctas_per_sm`, which caches the occupancy query: pass a
+// static of the launcher, one per kernel instantiation, starting at 0.  launch_persistent() then launches one CTA per
+// resident slot, never more CTAs than tiles.
+template <typename Kern>
+int persistent_ctas(Kern kern, int threads, int smem, int& ctas_per_sm) {
+  if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess) return (int)cudaGetLastError();
+  if (ctas_per_sm == 0) {
+    int occ = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, threads, smem) != cudaSuccess || occ < 1) occ = 1;
+    ctas_per_sm = occ;
+  }
+  return 0;
+}
+
+template <typename Kern, typename... Args>
+int launch_persistent(Kern kern, int threads, int smem, int ctas_per_sm, int64_t num_tiles, cudaStream_t s,
+                      const Args&... args) {
+  int64_t grid = persistent_sms() * ctas_per_sm;
+  if (grid > num_tiles) grid = num_tiles;
+  kern<<<(unsigned)grid, threads, smem, s>>>(args...);
+  count_launch();
+  return launch_status();
 }
 
 // ---------------------------------------------------------------- value-type traits
@@ -147,6 +177,50 @@ __device__ __forceinline__ T shfl_idx(unsigned mask, T v, int src, int width) {
 template <typename T>
 __device__ __forceinline__ T shfl_x(unsigned mask, T v, int lanemask) {
   return __shfl_xor_sync(mask, v, lanemask);
+}
+
+// Reduce NB per-lane partials across the LPR lanes of a group with a halving butterfly.
+// NB <= LPR: lane gl ends with the total of entry gl / (LPR/NB) in p[0].
+// NB >  LPR: lane gl ends with the totals of entries gl*(NB/LPR) + i in p[i], i < NB/LPR.
+template <typename Acc, int LPR, int NB>
+__device__ __forceinline__ void butterfly_reduce(Acc (&p)[NB], unsigned gmask, int gl) {
+  int width = NB;
+#pragma unroll
+  for (int s = LPR / 2; s >= 1; s >>= 1) {
+    if (width > 1) {
+      const int half = width / 2;
+      const bool upper = (gl & s) != 0;
+#pragma unroll
+      for (int i = 0; i < NB / 2; ++i) {
+        if (i < half) {
+          const Acc send = upper ? p[i] : p[i + half];
+          const Acc keep = upper ? p[i + half] : p[i];
+          p[i] = keep + shfl_x(gmask, send, s);
+        }
+      }
+      width = half;
+    } else {
+      p[0] += shfl_x(gmask, p[0], s);
+    }
+  }
+}
+
+// (elements per load, lanes per row, vectors per lane) of the row-split kernels: f(EPV, LPR, VPL) as
+// std::integral_constants.  `vec`: 128-bit loads of EPVF elements; otherwise scalar loads that honour any column stride.
+template <int EPVF, typename F>
+int with_rowsplit_lanes(bool vec, int64_t K, F&& f) {
+  if (vec) {
+    const int64_t kv = K / EPVF;  // vectors per row
+    if (kv <= 4) return f(Int<EPVF>{}, Int<4>{}, Int<1>{});
+    if (kv <= 8) return f(Int<EPVF>{}, Int<8>{}, Int<1>{});
+    if (kv <= 16) return f(Int<EPVF>{}, Int<16>{}, Int<1>{});
+    if (kv <= 32) return f(Int<EPVF>{}, Int<32>{}, Int<1>{});
+    if (kv <= 64) return f(Int<EPVF>{}, Int<32>{}, Int<2>{});
+    return f(Int<EPVF>{}, Int<32>{}, Int<4>{});  // K > 128 vectors: chunk loop inside
+  }
+  if (K == 1) return f(Int<1>{}, Int<1>{}, Int<1>{});
+  if (K <= 4) return f(Int<1>{}, Int<4>{}, Int<1>{});
+  return f(Int<1>{}, Int<32>{}, Int<1>{});
 }
 
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }

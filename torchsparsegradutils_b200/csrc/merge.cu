@@ -78,27 +78,23 @@ __device__ __forceinline__ void merge_search_smem(const I* rp, int64_t i0, int64
 }
 
 // ------------------------------------------------------------------------------------ shared memory
+// a tile holds at most MERGE_P row ends and MERGE_P entries; its rowptr slice one more (the row that ends after it)
 template <typename V, typename I, int VALS>
-struct MergeStage {
-  static constexpr int AI = 16 / (int)sizeof(I), AV = 16 / (int)sizeof(V);
-  alignas(16) I rp[MERGE_P + 2 + 2 * AI];
-  alignas(16) I col[MERGE_P + 2 * AI];
-  alignas(16) V val[VALS == 1 ? MERGE_P + 2 * AV : AV];
-  alignas(16) I prm[VALS == 2 ? MERGE_P + 2 * AI : AI];
-};
+using MergeStage = Stage<V, I, VALS, MERGE_P + 1, MERGE_P>;
 
+// Streams a tile's rowptr / colind / values (VALS as in TileCfg) into a stage; the tile's path coordinates are
+// (i0, j0) .. (i1, j1).
 template <typename V, typename I, int VALS>
 struct MergeProducer {
-  using Stage = MergeStage<V, I, VALS>;
   const I* rowptr; const I* colind; const V* vals; const I* perm;
   int64_t rowptr_len, nnz_len;
-  __device__ __forceinline__ void issue(Stage& st, uint64_t* bar, int64_t i0, int64_t j0, int64_t i1, int64_t j1) const {
-    using TP = TileProducer<V, I, 0>;
-    uint32_t tx = TP::template span<I>(st.rp, rowptr, i0, i1 + 2 < rowptr_len ? i1 + 2 : rowptr_len, rowptr_len, bar);
+  __device__ __forceinline__ void issue(MergeStage<V, I, VALS>& st, uint64_t* bar, int64_t i0, int64_t j0, int64_t i1,
+                                        int64_t j1) const {
+    uint32_t tx = bulk_span<I>(st.rp, rowptr, i0, i1 + 2 < rowptr_len ? i1 + 2 : rowptr_len, rowptr_len, bar);
     if (j1 > j0) {
-      tx += TP::template span<I>(st.col, colind, j0, j1, nnz_len, bar);
-      if constexpr (VALS == 1) tx += TP::template span<V>(st.val, vals, j0, j1, nnz_len, bar);
-      if constexpr (VALS == 2) tx += TP::template span<I>(st.prm, perm, j0, j1, nnz_len, bar);
+      tx += bulk_span<I>(st.col, colind, j0, j1, nnz_len, bar);
+      if constexpr (VALS == 1) tx += bulk_span<V>(st.val, vals, j0, j1, nnz_len, bar);
+      if constexpr (VALS == 2) tx += bulk_span<I>(st.prm, perm, j0, j1, nnz_len, bar);
     }
     mbar_expect_tx(bar, tx);
   }
@@ -440,14 +436,9 @@ static int launch_spmm_merge(const I* rowptr, const I* colind, const V* vals, co
   const bool exact = (K / EPV) == (int64_t)LPR * VPL;
   auto kern = exact ? spmm_merge_kernel<V, I, LPR, VPL, U, true, PERM> : spmm_merge_kernel<V, I, LPR, VPL, U, false, PERM>;
   const int smem = (int)sizeof(MergeSpmmSmem<V, I, PERM ? 2 : 1, LPR, VPL>);
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-  if (e != cudaSuccess) return (int)e;
-  int occ = 0;
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, 256, smem) != cudaSuccess || occ < 1) occ = 1;
-  int64_t grid = persistent_sms() * occ;
-  if (grid > num_tiles) grid = num_tiles;
-  kern<<<(unsigned)grid, 256, smem, s>>>(p, num_tiles);
-  count_launch();
+  static int ctas_per_sm[2] = {0, 0};
+  if (const int rc = persistent_ctas(kern, 256, smem, ctas_per_sm[exact])) return rc;
+  launch_persistent(kern, 256, smem, ctas_per_sm[exact], num_tiles, s, p, num_tiles);  // a failure shows in launch_status() below
   const int64_t fix_threads = num_tiles * LPR;
   spmm_merge_fixup_kernel<V, LPR, VPL><<<(unsigned)((fix_threads + 255) / 256), 256, 0, s>>>(p.carry, p.carry_row, num_tiles,
                                                                                             kpad, K, C, ldc);
@@ -460,9 +451,8 @@ size_t spmm_merge_workspace_bytes(int64_t rows, int64_t K, int64_t nnz, int val_
   const int esz = val_dtype == TSGU_F64 ? 8 : val_dtype == TSGU_BF16 ? 2 : 4;
   const int asz = val_dtype == TSGU_F64 ? 8 : 4;
   const int epv = 16 / esz;
-  int64_t kv = (K + epv - 1) / epv;  // vectors per row -> lane tiling used by the dispatcher
-  int64_t slots = kv <= 4 ? 4 : kv <= 8 ? 8 : kv <= 16 ? 16 : kv <= 32 ? 32 : kv <= 64 ? 64 : 128;  // = LPR*VPL in both lane tables
-  const int64_t kpad = slots * epv;
+  const int64_t kv = (K + epv - 1) / epv;  // vectors per row
+  const int64_t kpad = with_tile_lanes(kv, [](auto LPR, auto VPL) { return (int64_t)LPR * VPL; }) * epv;
   const size_t part_bytes = ((size_t)(num_tiles + 1) * 2 * sizeof(int64_t) + 255) / 256 * 256;
   const size_t row_bytes = ((size_t)num_tiles * 2 * sizeof(int64_t) + 255) / 256 * 256;
   return part_bytes + row_bytes + (size_t)num_tiles * 2 * kpad * asz;
@@ -472,19 +462,10 @@ size_t spmm_merge_workspace_bytes(int64_t rows, int64_t K, int64_t nnz, int val_
 template <typename V, typename I>
 int spmm_merge_dispatch(const I* rowptr, const I* colind, const V* vals, const I* perm, const V* B, V* C, int64_t rows,
                         int64_t K, int64_t nnz, int64_t b_rs, int64_t ldc, void* ws, size_t ws_bytes, cudaStream_t s) {
-  constexpr int EPVF = 16 / sizeof(V);
-  const int64_t kv = K / EPVF;
-#define TSGU_MERGE(LPR_, VPL_)                                                                                      \
-  return perm ? launch_spmm_merge<V, I, LPR_, VPL_, true>(rowptr, colind, vals, perm, B, C, rows, K, nnz, b_rs, ldc, ws, ws_bytes, s) \
-              : launch_spmm_merge<V, I, LPR_, VPL_, false>(rowptr, colind, vals, perm, B, C, rows, K, nnz, b_rs, ldc, ws, ws_bytes, s)
-  if (kv <= 4) TSGU_MERGE(4, 1);
-  if (kv <= 8) TSGU_MERGE(8, 1);
-  // 8-lane groups with 2-4 vectors per lane, as the tile kernels (config 4: 9.7 ms with 16/32-lane groups, 9.2 ms)
-  if (kv <= 16) TSGU_MERGE(8, 2);
-  if (kv <= 32) TSGU_MERGE(8, 4);
-  if (kv <= 64) TSGU_MERGE(16, 4);
-  TSGU_MERGE(32, 4);
-#undef TSGU_MERGE
+  return with_tile_lanes(K / (16 / (int)sizeof(V)), [&](auto LPR, auto VPL) {
+    return perm ? launch_spmm_merge<V, I, LPR, VPL, true>(rowptr, colind, vals, perm, B, C, rows, K, nnz, b_rs, ldc, ws, ws_bytes, s)
+                : launch_spmm_merge<V, I, LPR, VPL, false>(rowptr, colind, vals, perm, B, C, rows, K, nnz, b_rs, ldc, ws, ws_bytes, s);
+  });
 }
 
 #define TSGU_INST_MERGE(V, I)                                                                                     \
@@ -497,31 +478,6 @@ TSGU_INST_MERGE(double, int64_t)
 TSGU_INST_MERGE(__nv_bfloat16, int32_t)
 TSGU_INST_MERGE(__nv_bfloat16, int64_t)
 
-
-// Reduce NB per-lane partials across the LPR lanes of a group (see sddmm.cu): lane gl ends up with the
-// total of entry gl / (LPR/NB) in p[0].
-template <typename Acc, int LPR, int NB>
-__device__ __forceinline__ void butterfly_reduce_m(Acc (&p)[NB], unsigned gmask, int gl) {
-  int width = NB;
-#pragma unroll
-  for (int s = LPR / 2; s >= 1; s >>= 1) {
-    if (width > 1) {
-      const int half = width / 2;
-      const bool upper = (gl & s) != 0;
-#pragma unroll
-      for (int i = 0; i < NB / 2; ++i) {
-        if (i < half) {
-          const Acc send = upper ? p[i] : p[i + half];
-          const Acc keep = upper ? p[i + half] : p[i];
-          p[i] = keep + shfl_x(gmask, send, s);
-        }
-      }
-      width = half;
-    } else {
-      p[0] += shfl_x(gmask, p[0], s);
-    }
-  }
-}
 
 // ========================================================================================== SDDMM
 // Same decomposition; entries are independent, so there are no carries -- only the row of the
@@ -704,7 +660,7 @@ __global__ void __launch_bounds__(256, TSGU_MERGE_SDDMM_MINB) sddmm_merge_kernel
             }
           }
         }
-        butterfly_reduce_m<Acc, LPR, NB>(part, gmask, gl);
+        butterfly_reduce<Acc, LPR, NB>(part, gmask, gl);
         const int slot = gl / LPE;
         if ((gl % LPE) == 0 && slot < cnt) {
           const int64_t eo = tj0 + basel + slot;
@@ -735,15 +691,9 @@ static int launch_sddmm_merge(const MergeSddmmParams<V, I>& p0, void* ws, size_t
   const bool exact = (p.K / EPV) == (int64_t)LPR * VPL;
   auto kern = exact ? sddmm_merge_kernel<V, I, LPR, VPL, NB, U, true> : sddmm_merge_kernel<V, I, LPR, VPL, NB, U, false>;
   const int smem = (int)sizeof(MergeSddmmSmem<V, I>);
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-  if (e != cudaSuccess) return (int)e;
-  int occ = 0;
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, 256, smem) != cudaSuccess || occ < 1) occ = 1;
-  int64_t grid = persistent_sms() * occ;
-  if (grid > num_tiles) grid = num_tiles;
-  kern<<<(unsigned)grid, 256, smem, s>>>(p, num_tiles);
-  count_launch();
-  return launch_status();
+  static int ctas_per_sm[2] = {0, 0};
+  if (const int rc = persistent_ctas(kern, 256, smem, ctas_per_sm[exact])) return rc;
+  return launch_persistent(kern, 256, smem, ctas_per_sm[exact], num_tiles, s, p, num_tiles);
 }
 
 size_t sddmm_merge_workspace_bytes(int64_t rows, int64_t nnz) {
@@ -755,15 +705,9 @@ template <typename V, typename I>
 int sddmm_merge_dispatch(const I* rowptr, const I* colind, const I* out_index, const V* G, const V* B, V* out,
                          int64_t rows, int64_t K, int64_t nnz, int64_t g_rs, int64_t b_rs, void* ws, size_t ws_bytes,
                          cudaStream_t s) {
-  constexpr int EPVF = 16 / sizeof(V);
-  MergeSddmmParams<V, I> p{rowptr, colind, out_index, G, B, out, rows, K, nnz, g_rs, b_rs, nullptr};
-  const int64_t kv = K / EPVF;
-  if (kv <= 4) return launch_sddmm_merge<V, I, 4, 1>(p, ws, ws_bytes, s);
-  if (kv <= 8) return launch_sddmm_merge<V, I, 8, 1>(p, ws, ws_bytes, s);
-  if (kv <= 16) return launch_sddmm_merge<V, I, 8, 2>(p, ws, ws_bytes, s);
-  if (kv <= 32) return launch_sddmm_merge<V, I, 8, 4>(p, ws, ws_bytes, s);
-  if (kv <= 64) return launch_sddmm_merge<V, I, 16, 4>(p, ws, ws_bytes, s);
-  return launch_sddmm_merge<V, I, 32, 4>(p, ws, ws_bytes, s);
+  const MergeSddmmParams<V, I> p{rowptr, colind, out_index, G, B, out, rows, K, nnz, g_rs, b_rs, nullptr};
+  return with_tile_lanes(K / (16 / (int)sizeof(V)),
+                         [&](auto LPR, auto VPL) { return launch_sddmm_merge<V, I, LPR, VPL>(p, ws, ws_bytes, s); });
 }
 
 #define TSGU_INST_MERGE_SDDMM(V, I)                                                                              \

@@ -26,32 +26,6 @@ struct SddmmParams {
   int accumulate;  // tile kernel: out[dst] += dot (K processed in L2-sized slices)
 };
 
-// Reduce NB per-lane partials across the LPR lanes of a group with a halving butterfly.
-// NB <= LPR: lane gl ends with the total of entry gl / (LPR/NB) in p[0].
-// NB >  LPR: lane gl ends with the totals of entries gl*(NB/LPR) + i in p[i], i < NB/LPR.
-template <typename Acc, int LPR, int NB>
-__device__ __forceinline__ void butterfly_reduce(Acc (&p)[NB], unsigned gmask, int gl) {
-  int width = NB;
-#pragma unroll
-  for (int s = LPR / 2; s >= 1; s >>= 1) {
-    if (width > 1) {
-      const int half = width / 2;
-      const bool upper = (gl & s) != 0;
-#pragma unroll
-      for (int i = 0; i < NB / 2; ++i) {
-        if (i < half) {
-          const Acc send = upper ? p[i] : p[i + half];
-          const Acc keep = upper ? p[i + half] : p[i];
-          p[i] = keep + shfl_x(gmask, send, s);
-        }
-      }
-      width = half;
-    } else {
-      p[0] += shfl_x(gmask, p[0], s);
-    }
-  }
-}
-
 template <typename V, typename I, int EPV, int LPR, int VPL, int NB>
 __global__ void __launch_bounds__(256) sddmm_rowsplit_kernel(const SddmmParams<V, I> p) {
   using Acc = typename VT<V>::Acc;
@@ -154,7 +128,7 @@ __global__ void __launch_bounds__(256, TSGU_TILE_MINB(VPL)) sddmm_tile_kernel(co
   using Cfg = TileCfg<V, I, 0>;
   using Smem = typename Cfg::Smem;
   constexpr int EPV = 16 / sizeof(V);
-  constexpr int CAP = Cfg::CAP, AI = Cfg::ALN_I;
+  constexpr int CAP = Cfg::CAP, AI = Cfg::Stage::AI;
   constexpr int LPE = NB <= LPR ? LPR / NB : 1;  // lanes holding the same entry after the butterfly
   constexpr int RPL = NB <= LPR ? 1 : NB / LPR;  // results per lane after the butterfly
   constexpr int QC = (NB + LPR - 1) / LPR;       // column indices each lane holds per batch
@@ -328,35 +302,21 @@ static int launch_sddmm_tile(const SddmmParams<V, I>& p, int64_t nnz_total, cuda
   auto kern = exact ? sddmm_tile_kernel<V, I, LPR, VPL, NB, U, true> : sddmm_tile_kernel<V, I, LPR, VPL, NB, U, false>;
   const int smem = (int)sizeof(typename Cfg::Smem);
   static int ctas_per_sm[2] = {0, 0};
-  if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess) return (int)cudaGetLastError();
-  if (ctas_per_sm[exact] == 0) {
-    int occ = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, 256, smem) != cudaSuccess || occ < 1) occ = 1;
-    ctas_per_sm[exact] = occ;
-  }
+  if (const int rc = persistent_ctas(kern, 256, smem, ctas_per_sm[exact])) return rc;
   const int tile_rows = balance_tile_rows(
       pick_tile_rows(p.batch * p.n, nnz_total, Cfg::CAP, 256 / LPR, VPL == 1 ? 256 : TSGU_TILE_ROWS_DEFAULT), p.n, p.batch,
       nnz_total, Cfg::CAP, (int64_t)kNumSMs * ctas_per_sm[exact], 256 / LPR);
   const int64_t tiles_per_item = (p.n + tile_rows - 1) / tile_rows;
   const int64_t num_tiles = tiles_per_item * p.batch;
-  int64_t grid = persistent_sms() * ctas_per_sm[exact];
-  if (grid > num_tiles) grid = num_tiles;
   const int64_t rowptr_len = p.nnz_bstride > 0 ? p.batch * p.rowptr_bstride : p.batch * p.n + 1;
-  kern<<<(unsigned)grid, 256, smem, s>>>(p, tiles_per_item, num_tiles, rowptr_len, nnz_total, tile_rows);
-  count_launch();
-  return launch_status();
+  return launch_persistent(kern, 256, smem, ctas_per_sm[exact], num_tiles, s, p, tiles_per_item, num_tiles, rowptr_len,
+                           nnz_total, tile_rows);
 }
 
 template <typename V, typename I>
 static int sddmm_tile_dispatch(const SddmmParams<V, I>& p, int64_t nnz_total, cudaStream_t s) {
-  constexpr int EPVF = 16 / sizeof(V);
-  const int64_t kv = p.K / EPVF;
-  if (kv <= 4) return launch_sddmm_tile<V, I, 4, 1>(p, nnz_total, s);
-  if (kv <= 8) return launch_sddmm_tile<V, I, 8, 1>(p, nnz_total, s);
-  if (kv <= 16) return launch_sddmm_tile<V, I, 8, 2>(p, nnz_total, s);
-  if (kv <= 32) return launch_sddmm_tile<V, I, 8, 4>(p, nnz_total, s);
-  if (kv <= 64) return launch_sddmm_tile<V, I, 16, 4>(p, nnz_total, s);
-  return launch_sddmm_tile<V, I, 32, 4>(p, nnz_total, s);
+  return with_tile_lanes(p.K / (16 / (int)sizeof(V)),
+                         [&](auto LPR, auto VPL) { return launch_sddmm_tile<V, I, LPR, VPL>(p, nnz_total, s); });
 }
 
 template <typename V, typename I>
@@ -389,18 +349,7 @@ static int sddmm_dispatch(const SddmmParams<V, I>& p, int64_t m, int64_t nnz_tot
     }
     return sddmm_tile_dispatch<V, I>(p, nnz_total, s);
   }
-  if (vec_ok) {
-    const int64_t kv = p.K / EPVF;
-    if (kv <= 4) return launch_sddmm<V, I, EPVF, 4, 1>(p, s);
-    if (kv <= 8) return launch_sddmm<V, I, EPVF, 8, 1>(p, s);
-    if (kv <= 16) return launch_sddmm<V, I, EPVF, 16, 1>(p, s);
-    if (kv <= 32) return launch_sddmm<V, I, EPVF, 32, 1>(p, s);
-    if (kv <= 64) return launch_sddmm<V, I, EPVF, 32, 2>(p, s);
-    return launch_sddmm<V, I, EPVF, 32, 4>(p, s);
-  }
-  if (p.K == 1) return launch_sddmm<V, I, 1, 1, 1>(p, s);
-  if (p.K <= 4) return launch_sddmm<V, I, 1, 4, 1>(p, s);
-  return launch_sddmm<V, I, 1, 32, 1>(p, s);
+  return with_rowsplit_lanes<EPVF>(vec_ok, p.K, [&](auto EPV, auto LPR, auto VPL) { return launch_sddmm<V, I, EPV, LPR, VPL>(p, s); });
 }
 
 // ---------------------------------------------------------------------------------------------

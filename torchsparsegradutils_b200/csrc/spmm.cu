@@ -140,7 +140,7 @@ __global__ void __launch_bounds__(256, TSGU_TILE_MINB(VPL)) spmm_tile_kernel(con
   using Cfg = TileCfg<V, I, PERM ? 2 : 1>;
   using Smem = typename Cfg::Smem;
   constexpr int EPV = 16 / sizeof(V);
-  constexpr int CAP = Cfg::CAP, AI = Cfg::ALN_I, AV = Cfg::ALN_V;
+  constexpr int CAP = Cfg::CAP, AI = Cfg::Stage::AI, AV = Cfg::Stage::AV;
   extern __shared__ __align__(16) unsigned char smem_raw[];
   Smem& sm = *reinterpret_cast<Smem*>(smem_raw);
 
@@ -307,39 +307,21 @@ static int launch_tile(const SpmmParams<V, I>& p, int64_t nnz_total, cudaStream_
   auto kern = exact ? spmm_tile_kernel<V, I, LPR, VPL, U, true, PERM> : spmm_tile_kernel<V, I, LPR, VPL, U, false, PERM>;
   const int smem = (int)sizeof(typename Cfg::Smem);
   static int ctas_per_sm[2] = {0, 0};  // per instantiation; same answer on every B200 of the box
-  if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) != cudaSuccess) return (int)cudaGetLastError();
-  if (ctas_per_sm[exact] == 0) {
-    int occ = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, 256, smem) != cudaSuccess || occ < 1) occ = 1;
-    ctas_per_sm[exact] = occ;
-  }
+  if (const int rc = persistent_ctas(kern, 256, smem, ctas_per_sm[exact])) return rc;
   const int tile_rows = balance_tile_rows(pick_tile_rows(p.batch * p.n, nnz_total, Cfg::CAP, 256 / LPR), p.n, p.batch,
                                           nnz_total, Cfg::CAP, (int64_t)kNumSMs * ctas_per_sm[exact], 256 / LPR);
   const int64_t tiles_per_item = (p.n + tile_rows - 1) / tile_rows;
   const int64_t num_tiles = tiles_per_item * p.batch;
-  int64_t grid = persistent_sms() * ctas_per_sm[exact];
-  if (grid > num_tiles) grid = num_tiles;
   const int64_t rowptr_len = p.nnz_bstride > 0 ? p.batch * p.rowptr_bstride : p.batch * p.n + 1;
-  kern<<<(unsigned)grid, 256, smem, s>>>(p, tiles_per_item, num_tiles, rowptr_len, nnz_total, tile_rows);
-  count_launch();
-  return launch_status();
+  return launch_persistent(kern, 256, smem, ctas_per_sm[exact], num_tiles, s, p, tiles_per_item, num_tiles, rowptr_len,
+                           nnz_total, tile_rows);
 }
 
 template <typename V, typename I>
 static int spmm_tile_dispatch(const SpmmParams<V, I>& p, int64_t nnz_total, cudaStream_t s) {
-  constexpr int EPVF = 16 / sizeof(V);
-  const int64_t kv = p.K / EPVF;
-#define TSGU_TILE(LPR_, VPL_) \
-  return p.perm ? launch_tile<V, I, LPR_, VPL_, true>(p, nnz_total, s) : launch_tile<V, I, LPR_, VPL_, false>(p, nnz_total, s)
-  // narrower lane groups with more vectors per lane serve several rows per warp instruction, which
-  // divides the shuffle (col / val broadcast) traffic on the LSU return path (DESIGN.md section 3.1)
-  if (kv <= 4) TSGU_TILE(4, 1);
-  if (kv <= 8) TSGU_TILE(8, 1);
-  if (kv <= 16) TSGU_TILE(8, 2);
-  if (kv <= 32) TSGU_TILE(8, 4);
-  if (kv <= 64) TSGU_TILE(16, 4);
-  TSGU_TILE(32, 4);
-#undef TSGU_TILE
+  return with_tile_lanes(p.K / (16 / (int)sizeof(V)), [&](auto LPR, auto VPL) {
+    return p.perm ? launch_tile<V, I, LPR, VPL, true>(p, nnz_total, s) : launch_tile<V, I, LPR, VPL, false>(p, nnz_total, s);
+  });
 }
 
 template <typename V, typename I>
@@ -373,21 +355,23 @@ static int spmm_dispatch(const SpmmParams<V, I>& p, int64_t m, int64_t nnz_total
     }
     return spmm_tile_dispatch<V, I>(p, nnz_total, s);
   }
-  if (vec_ok) {
-    const int64_t kv = p.K / EPVF;  // vectors per row
-    if (kv <= 4) return launch_rowsplit<V, I, EPVF, 4, 1>(p, s);
-    if (kv <= 8) return launch_rowsplit<V, I, EPVF, 8, 1>(p, s);
-    if (kv <= 16) return launch_rowsplit<V, I, EPVF, 16, 1>(p, s);
-    if (kv <= 32) return launch_rowsplit<V, I, EPVF, 32, 1>(p, s);
-    if (kv <= 64) return launch_rowsplit<V, I, EPVF, 32, 2>(p, s);
-    return launch_rowsplit<V, I, EPVF, 32, 4>(p, s);  // K > 128 vectors: chunk loop inside
-  }
-  if (p.K == 1) return launch_rowsplit<V, I, 1, 1, 1>(p, s);
-  if (p.K <= 4) return launch_rowsplit<V, I, 1, 4, 1>(p, s);
-  return launch_rowsplit<V, I, 1, 32, 1>(p, s);
+  return with_rowsplit_lanes<EPVF>(vec_ok, p.K, [&](auto EPV, auto LPR, auto VPL) { return launch_rowsplit<V, I, EPV, LPR, VPL>(p, s); });
 }
 
 }  // namespace tsgu
+
+// the shared body of the two SpMM entry points
+static int spmm_csr(const void* rowptr, const void* colind, const void* vals, const void* perm, const void* row_map, const void* B,
+                    void* C, int64_t batch, int64_t n, int64_t m, int64_t K, int64_t rowptr_bstride, int64_t nnz_bstride,
+                    int64_t nnz_total, int64_t b_bs, int64_t b_rs, int64_t b_cs, int64_t c_bs, int64_t ldc, int val_dtype,
+                    int idx_dtype, int algo, void* workspace, size_t workspace_bytes, void* stream) {
+  TSGU_DISPATCH_VAL(val_dtype, TSGU_DISPATCH_IDX(idx_dtype, {
+    const tsgu::SpmmParams<V, I> p{(const I*)rowptr, (const I*)colind, (const V*)vals, (const I*)perm, (const V*)B, (V*)C,
+                                   batch, n, K, rowptr_bstride, nnz_bstride, b_bs, b_rs, b_cs, c_bs, ldc, (const I*)row_map};
+    return tsgu::spmm_dispatch<V, I>(p, m, nnz_total, algo, workspace, workspace_bytes, tsgu::as_stream(stream));
+  }));
+  return 0;
+}
 
 extern "C" int tsgu_spmm_csr(const void* rowptr, const void* colind, const void* vals, const void* perm,
                              const void* B, void* C, int64_t batch, int64_t n, int64_t m, int64_t K,
@@ -401,17 +385,8 @@ extern "C" int tsgu_spmm_csr(const void* rowptr, const void* colind, const void*
     if (family != TSGU_ALGO_AUTO && family != TSGU_ALGO_ROWSPLIT && family != TSGU_ALGO_MERGE) return TSGU_ERR_ALGO;
   }
   if (batch == 0 || n == 0 || K == 0) return 0;
-  TSGU_DISPATCH_VAL(val_dtype, TSGU_DISPATCH_IDX(idx_dtype, {
-    tsgu::SpmmParams<V, I> p;
-    p.rowptr = (const I*)rowptr; p.colind = (const I*)colind; p.vals = (const V*)vals;
-    p.perm = (const I*)perm; p.B = (const V*)B; p.C = (V*)C;
-    p.batch = batch; p.n = n; p.K = K;
-    p.rowptr_bstride = rowptr_bstride; p.nnz_bstride = nnz_bstride;
-    p.b_bs = b_bs; p.b_rs = b_rs; p.b_cs = b_cs; p.c_bs = c_bs; p.ldc = ldc;
-    p.row_map = nullptr;
-    return tsgu::spmm_dispatch<V, I>(p, m, nnz_total, algo, workspace, workspace_bytes, tsgu::as_stream(stream));
-  }));
-  return 0;
+  return spmm_csr(rowptr, colind, vals, perm, nullptr, B, C, batch, n, m, K, rowptr_bstride, nnz_bstride, nnz_total, b_bs,
+                  b_rs, b_cs, c_bs, ldc, val_dtype, idx_dtype, algo, workspace, workspace_bytes, stream);
 }
 
 extern "C" int tsgu_spmm_csr_rowmap(const void* rowptr, const void* colind, const void* vals, const void* perm,
@@ -423,17 +398,8 @@ extern "C" int tsgu_spmm_csr_rowmap(const void* rowptr, const void* colind, cons
   const int family = algo & ~TSGU_ALGO_FLAG_KSLICE;
   if (family != TSGU_ALGO_AUTO && family != TSGU_ALGO_ROWSPLIT) return TSGU_ERR_ALGO;  // merge-path has no row map
   if (batch == 0 || n == 0 || K == 0) return 0;
-  TSGU_DISPATCH_VAL(val_dtype, TSGU_DISPATCH_IDX(idx_dtype, {
-    tsgu::SpmmParams<V, I> p;
-    p.rowptr = (const I*)rowptr; p.colind = (const I*)colind; p.vals = (const V*)vals;
-    p.perm = (const I*)perm; p.B = (const V*)B; p.C = (V*)C;
-    p.batch = batch; p.n = n; p.K = K;
-    p.rowptr_bstride = rowptr_bstride; p.nnz_bstride = nnz_bstride;
-    p.b_bs = b_bs; p.b_rs = b_rs; p.b_cs = b_cs; p.c_bs = c_bs; p.ldc = ldc;
-    p.row_map = (const I*)row_map;
-    return tsgu::spmm_dispatch<V, I>(p, m, nnz_total, algo, nullptr, 0, tsgu::as_stream(stream));
-  }));
-  return 0;
+  return spmm_csr(rowptr, colind, vals, perm, row_map, B, C, batch, n, m, K, rowptr_bstride, nnz_bstride, nnz_total, b_bs,
+                  b_rs, b_cs, c_bs, ldc, val_dtype, idx_dtype, algo, nullptr, 0, stream);
 }
 
 extern "C" size_t tsgu_spmm_workspace_bytes(int64_t batch, int64_t n, int64_t K, int64_t nnz_total,

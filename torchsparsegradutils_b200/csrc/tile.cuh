@@ -63,6 +63,17 @@ __device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t by
 }
 
 // ------------------------------------------------------------------ tile geometry
+// One pipeline stage: the rowptr slice (ROWS + 1 entries) and up to CAP entries of colind and of the values
+// (VALS == 1) or of a value permutation (VALS == 2), each with room for the 16-B alignment shift of its first element.
+template <typename V, typename I, int VALS, int ROWS, int CAP>
+struct Stage {
+  static constexpr int AI = 16 / (int)sizeof(I), AV = 16 / (int)sizeof(V);
+  alignas(16) I rp[ROWS + 1 + 2 * AI];
+  alignas(16) I col[CAP + 2 * AI];
+  alignas(16) V val[VALS == 1 ? CAP + 2 * AV : AV];
+  alignas(16) I prm[VALS == 2 ? CAP + 2 * AI : AI];
+};
+
 // VALS: 0 = pattern only (SDDMM), 1 = values staged (SpMM), 2 = a value permutation staged instead
 // (SpMM over a transposed / COO-derived structure: the value of entry e is vals[perm[e]]).
 template <typename V, typename I, int VALS>
@@ -70,15 +81,8 @@ struct TileCfg {
   static constexpr int TILE_ROWS = TSGU_TILE_ROWS;
   // entries of colind / vals staged per tile: 32 KB per stage (4096 for fp32 + int32)
   static constexpr int CAP = (TSGU_TILE_STAGE_BYTES / (int)(sizeof(I) + (VALS == 1 ? sizeof(V) : VALS == 2 ? sizeof(I) : 0))) & ~15;
-  static constexpr int ALN_I = 16 / (int)sizeof(I);
-  static constexpr int ALN_V = 16 / (int)sizeof(V);
   static constexpr int STAGES = 2;
-  struct Stage {
-    alignas(16) I rp[TILE_ROWS + 1 + 2 * ALN_I];
-    alignas(16) I col[CAP + 2 * ALN_I];
-    alignas(16) V val[VALS == 1 ? CAP + 2 * ALN_V : ALN_V];
-    alignas(16) I prm[VALS == 2 ? CAP + 2 * ALN_I : ALN_I];
-  };
+  using Stage = tsgu::Stage<V, I, VALS, TILE_ROWS, CAP>;
   struct Smem {
     Stage st[STAGES];
     alignas(8) uint64_t full[STAGES];
@@ -142,8 +146,25 @@ __device__ __forceinline__ TileCoord tile_coord(int64_t t, int64_t tiles_per_ite
 }
 
 // ------------------------------------------------------------------ producer (one elected thread)
-// Streams rowptr[r0..r1], colind[s..e) and (WITH_VALS) vals[s..e) of a tile into a stage so that
-// element `lo` of each global array lands at dst[lo % ALN] (bulk copies need 16-B aligned ends).
+// Copies src[lo, hi) into dst so that element `lo` lands at dst[lo % A], A = 16 B / sizeof(T) (bulk copies need
+// 16-B aligned ends); returns the bytes the bulk copy will complete on `bar`.
+template <typename T>
+__device__ __forceinline__ uint32_t bulk_span(T* dst, const T* src, int64_t lo, int64_t hi, int64_t len, uint64_t* bar) {
+  constexpr int64_t A = 16 / (int64_t)sizeof(T);
+  const int64_t lo_al = lo & ~(A - 1);
+  int64_t hi_al = (hi + A - 1) & ~(A - 1);
+  const int64_t len_dn = len & ~(A - 1);
+  if (hi_al > len_dn) {  // the 16-B vector holding the array's ragged end is copied element-wise
+    for (int64_t k = (lo > len_dn ? lo : len_dn); k < hi; ++k) dst[k - lo_al] = src[k];
+    hi_al = len_dn;
+  }
+  if (hi_al <= lo_al) return 0u;
+  const uint32_t bytes = (uint32_t)((hi_al - lo_al) * (int64_t)sizeof(T));
+  bulk_g2s(dst, src + lo_al, bytes, bar);
+  return bytes;
+}
+
+// Streams rowptr[r0..r1], colind[s..e) and the values or their permutation (VALS) of a row tile into a stage.
 template <typename V, typename I, int VALS>
 struct TileProducer {
   using Cfg = TileCfg<V, I, VALS>;
@@ -161,32 +182,15 @@ struct TileProducer {
     e_abs = (int64_t)__ldg(rp + c.rows) + c.item * nnz_bstride;
   }
 
-  template <typename T>
-  __device__ __forceinline__ static uint32_t span(T* dst, const T* src, int64_t lo, int64_t hi, int64_t len,
-                                                  uint64_t* bar) {
-    constexpr int64_t A = 16 / (int64_t)sizeof(T);
-    const int64_t lo_al = lo & ~(A - 1);
-    int64_t hi_al = (hi + A - 1) & ~(A - 1);
-    const int64_t len_dn = len & ~(A - 1);
-    if (hi_al > len_dn) {  // the 16-B vector holding the array's ragged end is copied element-wise
-      for (int64_t k = (lo > len_dn ? lo : len_dn); k < hi; ++k) dst[k - lo_al] = src[k];
-      hi_al = len_dn;
-    }
-    if (hi_al <= lo_al) return 0u;
-    const uint32_t bytes = (uint32_t)((hi_al - lo_al) * (int64_t)sizeof(T));
-    bulk_g2s(dst, src + lo_al, bytes, bar);
-    return bytes;
-  }
-
   __device__ __forceinline__ void issue(typename Cfg::Stage& st, uint64_t* bar, int64_t t, int64_t s_abs,
                                         int64_t e_abs) const {
     const TileCoord c = tile_coord(t, tiles_per_item, n, tile_rows);
     const int64_t rp_lo = c.item * rowptr_bstride + c.r0;
-    uint32_t tx = span<I>(st.rp, rowptr, rp_lo, rp_lo + c.rows + 1, rowptr_len, bar);
+    uint32_t tx = bulk_span<I>(st.rp, rowptr, rp_lo, rp_lo + c.rows + 1, rowptr_len, bar);
     if ((e_abs - s_abs) <= Cfg::CAP && e_abs > s_abs) {
-      tx += span<I>(st.col, colind, s_abs, e_abs, nnz_len, bar);
-      if constexpr (VALS == 1) tx += span<V>(st.val, vals, s_abs, e_abs, nnz_len, bar);
-      if constexpr (VALS == 2) tx += span<I>(st.prm, perm, s_abs, e_abs, nnz_len, bar);
+      tx += bulk_span<I>(st.col, colind, s_abs, e_abs, nnz_len, bar);
+      if constexpr (VALS == 1) tx += bulk_span<V>(st.val, vals, s_abs, e_abs, nnz_len, bar);
+      if constexpr (VALS == 2) tx += bulk_span<I>(st.prm, perm, s_abs, e_abs, nnz_len, bar);
     }
     // arrive.expect_tx after the copies were issued is fine (the phase cannot complete before this
     // arrival) and, having release semantics, it also publishes the element-wise tail stores above
@@ -194,15 +198,19 @@ struct TileProducer {
   }
 };
 
-// Description of where a tile's slices landed in a stage (every thread recomputes it from the rowptr
-// slice in shared memory; nothing but the data itself is communicated).
-struct TileView {
-  int rp_shift;     // rp[rp_shift + k] = rowptr[r0 + k]
-  int64_t s_abs;    // absolute index of the tile's first stored entry
-  int64_t e_abs;    // one past its last entry
-  int col_shift;    // col[col_shift + (e - s_abs)] = colind[e]
-  int val_shift;
-  bool staged;      // colind / vals are in shared memory (tile fits CAP); else read them from global
-};
+// ------------------------------------------------------------------ lane table
+// (lanes per row, 128-bit vectors per lane) of the staged kernels, row-tile and merge-path, for kv vectors per dense
+// row: f(LPR, VPL) as std::integral_constants.  Narrower lane groups with more vectors per lane serve several rows per
+// warp instruction, which divides the shuffle (col / val broadcast) traffic on the LSU return path (DESIGN.md
+// section 3.1); merge-path config 4: 9.7 ms with 16/32-lane groups, 9.2 ms with this table.
+template <typename F>
+inline auto with_tile_lanes(int64_t kv, F&& f) {
+  if (kv <= 4) return f(Int<4>{}, Int<1>{});
+  if (kv <= 8) return f(Int<8>{}, Int<1>{});
+  if (kv <= 16) return f(Int<8>{}, Int<2>{});
+  if (kv <= 32) return f(Int<8>{}, Int<4>{});
+  if (kv <= 64) return f(Int<16>{}, Int<4>{});
+  return f(Int<32>{}, Int<4>{});
+}
 
 }  // namespace tsgu

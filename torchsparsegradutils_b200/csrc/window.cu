@@ -313,7 +313,6 @@ __device__ __forceinline__ void win_fetch_info(const WinParams<V, I>& p, WinInfo
 template <typename V, typename I, int ROWB, bool WITH_VALS>
 __device__ __forceinline__ void win_produce(const WinParams<V, I>& p, WinStage<V, I, ROWB, !WITH_VALS>& st, uint64_t* bar,
                                             const WinTileInfo& ti, int item, int r0, int rows, int lane) {
-  using TP = TileProducer<V, I, 0>;
   uint32_t tx = 0;
   if (lane < ti.nruns) {
     const uint32_t slot = ti.sl & 0xffffu, len = ti.sl >> 16;
@@ -329,10 +328,10 @@ __device__ __forceinline__ void win_produce(const WinParams<V, I>& p, WinStage<V
   }
   if (lane == 0) {
     const int64_t rp_lo = (int64_t)item * p.rowptr_bstride + r0;
-    tx += TP::template span<I>(st.rp, p.rowptr, rp_lo, rp_lo + rows + 1, p.rowptr_len, bar);
+    tx += bulk_span<I>(st.rp, p.rowptr, rp_lo, rp_lo + rows + 1, p.rowptr_len, bar);
     if (ti.e_abs > ti.s_abs) {
-      tx += TP::template span<uint16_t>(st.lcol, p.lcol, ti.s_abs, ti.e_abs, p.nnz_len, bar);
-      if constexpr (WITH_VALS) tx += TP::template span<V>(st.val, p.vals, ti.s_abs, ti.e_abs, p.nnz_len, bar);
+      tx += bulk_span<uint16_t>(st.lcol, p.lcol, ti.s_abs, ti.e_abs, p.nnz_len, bar);
+      if constexpr (WITH_VALS) tx += bulk_span<V>(st.val, p.vals, ti.s_abs, ti.e_abs, p.nnz_len, bar);
     }
   }
   if constexpr (!WITH_VALS) {  // SDDMM: the tile's rows of the upstream gradient (consecutive rows)
@@ -635,35 +634,26 @@ __global__ void __launch_bounds__(TSGU_WIN_CW * 32 + 32) sddmm_window_kernel(con
 }
 
 // ---------------------------------------------------------------------------------------- launch
-template <typename Kern, typename Params>
-static int win_launch(Kern kern, int smem, int64_t num_tiles, cudaStream_t s, int* occ_cache, const Params& params) {
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-  if (e != cudaSuccess) return (int)e;
-  if (*occ_cache == 0) {
-    int occ = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, TSGU_WIN_CW * 32 + 32, smem) != cudaSuccess || occ < 1) occ = 1;
-    *occ_cache = occ;
-  }
-  int64_t grid = persistent_sms() * *occ_cache;
-  if (grid > num_tiles) grid = num_tiles;
-  kern<<<(unsigned)grid, TSGU_WIN_CW * 32 + 32, smem, s>>>(params);
-  count_launch();
-  return launch_status();
+// the window kernels' persistent launch (producer warp + TSGU_WIN_CW consumer warps per CTA)
+template <typename Kern, typename V, typename I>
+static int win_launch(Kern kern, int smem, int& ctas_per_sm, const WinParams<V, I>& p, cudaStream_t s) {
+  if (const int rc = persistent_ctas(kern, TSGU_WIN_CW * 32 + 32, smem, ctas_per_sm)) return rc;
+  return launch_persistent(kern, TSGU_WIN_CW * 32 + 32, smem, ctas_per_sm, p.num_tiles, s, p);
 }
 
 template <typename V, typename I, int LPR, int VPL>
 static int launch_spmm_window(const WinParams<V, I>& p, cudaStream_t s) {
   constexpr int ROWB = LPR * VPL * 16;
   constexpr int U = VPL >= 4 ? 2 : (VPL == 2 ? 4 : 8);
-  static int occ = 0;
-  return win_launch(spmm_window_kernel<V, I, LPR, VPL, U>, (int)sizeof(WinSmem<V, I, ROWB>), p.num_tiles, s, &occ, p);
+  static int ctas_per_sm = 0;
+  return win_launch(spmm_window_kernel<V, I, LPR, VPL, U>, (int)sizeof(WinSmem<V, I, ROWB>), ctas_per_sm, p, s);
 }
 
 template <typename V, typename I, int LPR, int VPL>
 static int launch_sddmm_window(const WinParams<V, I>& p, cudaStream_t s) {
   constexpr int ROWB = LPR * VPL * 16;
-  static int occ = 0;
-  return win_launch(sddmm_window_kernel<V, I, LPR, VPL>, (int)sizeof(WinSmem<V, I, ROWB, true>), p.num_tiles, s, &occ, p);
+  static int ctas_per_sm = 0;
+  return win_launch(sddmm_window_kernel<V, I, LPR, VPL>, (int)sizeof(WinSmem<V, I, ROWB, true>), ctas_per_sm, p, s);
 }
 
 template <typename V, typename I>
