@@ -15,7 +15,7 @@ NAME=$1; FILES=$2; shift; shift
 TMP=${TMPDIR:-/tmp}
 mkdir -p "$ROOT/variants_tmp"
 OBJS=""
-for f in api spmm sddmm index merge window; do
+for f in api spmm sddmm index merge window trisolve; do
   if [[ " $FILES " == *" $f "* ]]; then
     nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -Xcompiler -fPIC,-fvisibility=hidden \
       --expt-relaxed-constexpr -Xptxas -v -DTSGU_BUILD "$@" -c $f.cu -o $TMP/${f}_$NAME.o > $TMP/${f}_$NAME.log 2>&1 &
